@@ -9,7 +9,8 @@ all: lib cli oracle sim
 
 lib: rsicnv_b200/librsigpu.so
 rsicnv_b200/librsigpu.so: $(CSRC)/rsigpu.cu $(HDRS)
-	$(NVCC) $(NVFLAGS) -shared $< -o $@ 2> build_ptxas.log || (cat build_ptxas.log; exit 1)
+	@mkdir -p build
+	$(NVCC) $(NVFLAGS) -shared $< -o $@ 2> build/ptxas.log || (cat build/ptxas.log; exit 1)
 
 # the host program (argv, BGZF/BAM, FASTA, depth text, output table) over the C ABI
 cli: rsicnv_b200/bin/rsicnv
@@ -32,5 +33,5 @@ ref:
 	$(MAKE) -f oracle/Makefile.ref -j8
 
 clean:
-	rm -rf rsicnv_b200/bin rsicnv_b200/librsigpu.so oracle/librsi_oracle.so tests/hostsim/*.so build_ptxas.log
+	rm -rf rsicnv_b200/bin rsicnv_b200/librsigpu.so oracle/librsi_oracle.so tests/hostsim/*.so build/ptxas.log
 .PHONY: all lib oracle sim ref clean

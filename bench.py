@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Gbases/s of the B200-native `rsicnv rsi` depth -> CNV-call path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload wg|chr19_bam|chr19_depth]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload wg|chr19_bam|chr19_depth] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs):
   wg          (default; configs[2]) a b37-shaped genome -- 24 contigs in b37 proportions at --genome-scale (default 1/4: 774 Mbp,
@@ -257,6 +257,28 @@ def run_reference_arm(a, config, bam):
     return 0
 
 
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, per_contig: list) -> None:
+    """per_contig[i] = (statistics, calls) of contig i in header order -> DIR/contig_<statistic>.npy (one value per contig),
+    DIR/call_<field>.npy (one value per call, contigs in header order) and DIR/call_contig.npy (each call's contig index).
+    Above DUMP_CAP_BYTES in all, the call files hold a fixed seeded sample of the calls (same rows in every file, in order)."""
+    from rsicnv_b200 import api
+    os.makedirs(path, exist_ok=True)
+    for k in per_contig[0][0]:
+        np.save(os.path.join(path, f"contig_{k}.npy"), np.array([s[k] for s, _ in per_contig], np.float64))
+    calls = [(i, c) for i, (_, cs) in enumerate(per_contig) for c in cs]
+    fields = [n for n, _ in api.Cnv._fields_ if n != "pad_"]
+    room = (DUMP_CAP_BYTES - (1 << 16) - 8 * len(per_contig) * len(per_contig[0][0])) // (8 * (len(fields) + 1))
+    if len(calls) > room:
+        keep = np.sort(np.random.default_rng(0).choice(len(calls), room, replace=False))
+        calls = [calls[j] for j in keep]
+    np.save(os.path.join(path, "call_contig.npy"), np.array([i for i, _ in calls], np.float64))
+    for k in fields:
+        np.save(os.path.join(path, f"call_{k}.npy"), np.array([c[k] for _, c in calls], np.float64))
+
+
 # ------------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -274,8 +296,12 @@ def main():
     ap.add_argument("--e2e-batch-mb", type=int, default=1000, help="e2e leg: compressed MiB of BAM one decoder feed takes (the contigs of a batch are inflated by one launch; "
                                                                       "a feed holds at most 2 GiB compressed and, here, 10 GiB decoded)")
     ap.add_argument("--no-cli", action="store_true", help="skip the CLI / one-core reference comparison at the end (N=1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the device-resident leg returned as DIR/<name>.npy "
+                                                          "(float64): every call's fields, in header order, and each contig's statistics")
     a = ap.parse_args()
-    rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes what this project's path computed: it needs --impl ours")
+    rank =int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     bam = a.workload != "chr19_depth"
     K = max(1, a.inflight)
     if a.workload == "wg":
@@ -404,10 +430,17 @@ def main():
     stages = ctx_of[big].stage_ms() if big is not None else {}
     # the table (rows of every contig, header order) -> one hash: equal at every N, since sharding must not change a single byte
     rows = {}
+    outputs = {}
     for i in mine:
         st = ctx_of[i].chr_stats()
         rows[i] = [api.format_row(ctx_of[i].lib, bufs[i][j], names[i], st.rdmedian, st.rdsd) for j in range(ncalls[i])]
+        if a.dump_outputs:
+            outputs[i] = [({n: getattr(st, n) for n, _ in api.ChrStats._fields_ if n != "reserved_"}, [bufs[i][j].as_dict() for j in range(ncalls[i])])]
     table = shard.gather_rows(rows, len(lens), rank, world)
+    if a.dump_outputs:
+        dump = shard.gather_rows(outputs, len(lens), rank, world)
+        if rank == 0:
+            dump_outputs(a.dump_outputs, dump)
     # ---- per-kernel device times on this rank's largest contig (extra profiled steps, CUDA events around every launch on the context's stream)
     prof = []
     if big is not None:

@@ -492,6 +492,95 @@ def write_bam_aligned(path: str, name: str, L: int, reads: dict, level: int = 1,
     return dict(rec_off=rec_off, blk_end=np.asarray(blk_end, np.int64), blk_rec_end=np.asarray(blk_rec_end, np.int64))
 
 
+def write_bai(bam_path: str) -> None:
+    """<bam_path>.bai for a coordinate-sorted BGZF/BAM file (SAM spec 5.2, laid out as samtools-0.1.18's bam_index_build
+    writes it): per reference one chunk per run of records with the same bin (adjacent chunks of a bin that meet in one BGZF
+    block merged), the pseudo-bin 37450 (file range of the reference, mapped / unmapped counts) and the 16 kbp linear index;
+    the count of unplaced records at the end.  Lets the indexed routes of the CLI run on the files write_bam produces."""
+    import struct
+    import zlib
+    raw = np.fromfile(bam_path, np.uint8)
+    blocks, foffs, dstarts = [], [], []
+    off = dlen = 0
+    while off < len(raw):
+        xlen = int(raw[off + 10]) | int(raw[off + 11]) << 8
+        bsize = (int(raw[off + 16]) | int(raw[off + 17]) << 8) + 1
+        blk = zlib.decompress(raw[off + 12 + xlen:off + bsize - 8].tobytes(), -15)
+        blocks.append(blk); foffs.append(off); dstarts.append(dlen)
+        off += bsize; dlen += len(blk)
+    dec = b"".join(blocks)
+    d = np.frombuffer(dec, np.uint8)
+    foffs = np.asarray(foffs, np.int64); dstarts = np.asarray(dstarts, np.int64)
+
+    def i32(at):
+        return (d[at].astype(np.int64) | d[at + 1].astype(np.int64) << 8 | d[at + 2].astype(np.int64) << 16 |
+                d[at + 3].astype(np.int64) << 24).astype(np.uint32).astype(np.int64)
+
+    l_text = struct.unpack_from("<i", dec, 4)[0]
+    n_ref = struct.unpack_from("<i", dec, 8 + l_text)[0]
+    p = 12 + l_text
+    for _ in range(n_ref):
+        p += 8 + struct.unpack_from("<i", dec, p)[0]
+    starts = []
+    while p < len(dec):
+        starts.append(p)
+        p += 4 + struct.unpack_from("<i", dec, p)[0]
+    s = np.asarray(starts + [len(dec)], np.int64)
+    k = np.searchsorted(dstarts, s, side="right") - 1           # the block a decoded offset lies in (its end: the next block)
+    voff = (foffs[k] << 16) | (s - dstarts[k])
+    s = s[:-1]
+    tid = i32(s + 4).astype(np.int32).astype(np.int64); pos = i32(s + 8).astype(np.int32).astype(np.int64)
+    bmn = i32(s + 12); fnc = i32(s + 16)
+    rbin = bmn >> 16; l_name = bmn & 0xff; flag = fnc >> 16; ncig = fnc & 0xffff
+    # alignment end (bam_calend): sum of M / D / N lengths; an end <= pos counts as pos + 1
+    cs = s + 36 + l_name
+    tot = int(ncig.sum())
+    ci = np.repeat(cs, ncig) + 4 * (np.arange(tot) - np.repeat(np.cumsum(ncig) - ncig, ncig))
+    cw = i32(ci) if tot else np.zeros(0, np.int64)
+    rl = np.where(np.isin(cw & 15, (0, 2, 3)), cw >> 4, 0)
+    end = pos + np.add.reduceat(rl, np.minimum(np.cumsum(ncig) - ncig, tot - 1)) * (ncig > 0) if tot else pos.copy()
+    end = np.maximum(end, pos + 1)
+    out = bytearray(b"BAI\x01") + struct.pack("<i", n_ref)
+    for r in range(n_ref):
+        idx = np.flatnonzero(tid == r)
+        if not len(idx):
+            out += struct.pack("<ii", 0, 0)
+            continue
+        beg, fin = voff[idx], voff[idx + 1]
+        cut = np.flatnonzero(np.diff(rbin[idx]) != 0) + 1       # runs of records with the same bin
+        rs = np.concatenate(([0], cut)); re = np.concatenate((cut, [len(idx)])) - 1
+        chunks: dict[int, list[list[int]]] = {}
+        for a, b in zip(rs, re):
+            lst = chunks.setdefault(int(rbin[idx[a]]), [])
+            u, v = int(beg[a]), int(fin[b])
+            if lst and lst[-1][1] >> 16 == u >> 16:
+                lst[-1][1] = v
+            else:
+                lst.append([u, v])
+        nmap = int(((flag[idx] & 4) == 0).sum())
+        chunks[37450] = [[int(beg[0]), int(fin[-1])], [nmap, len(idx) - nmap]]
+        out += struct.pack("<i", len(chunks))
+        for b in sorted(chunks):
+            out += struct.pack("<Ii", b, len(chunks[b]))
+            for u, v in chunks[b]:
+                out += struct.pack("<QQ", u, v)
+        w0 = pos[idx] >> 14; w1 = (end[idx] - 1) >> 14
+        nw = int(w1.max()) + 1
+        lin = np.full(nw, np.iinfo(np.int64).max, np.int64)
+        nwr = w1 - w0 + 1
+        np.minimum.at(lin, np.repeat(w0, nwr) + (np.arange(int(nwr.sum())) - np.repeat(np.cumsum(nwr) - nwr, nwr)), np.repeat(beg, nwr))
+        lin[lin == np.iinfo(np.int64).max] = 0
+        for j in range(1, nw):
+            if lin[j] == 0:
+                lin[j] = lin[j - 1]
+        out += struct.pack("<i", nw) + lin.astype("<u8").tobytes()
+    n_no_coor = int((tid < 0).sum())
+    if n_no_coor:
+        out += struct.pack("<Q", n_no_coor)
+    with open(bam_path + ".bai", "wb") as f:
+        f.write(bytes(out))
+
+
 def _reg2bin(beg, end):
     """UCSC binning (samtools bam.h:bam_reg2bin), vectorised"""
     end = end - 1

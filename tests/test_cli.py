@@ -1,6 +1,8 @@
 """The C++ host program (rsicnv_b200/bin/rsicnv): BGZF/BAM decoding and argument handling without a GPU;
 with a GPU, the whole CLI against the unmodified reference CLI on the same files (tables must be identical
 apart from the `#input` line, which echoes the path)."""
+import hashlib
+import json
 import os
 import subprocess
 
@@ -118,6 +120,121 @@ def test_cli_depth_file_matches_reference(cli, tmp_path):
     assert log_lines(str(tmp_path / "ours.txt.log"), str(tmp_path / "ours.txt")) == log_lines(str(tmp_path / "ref.txt.log"), str(tmp_path / "ref.txt"))
 
 
+GOLD = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_vectors.json")))
+
+
+def _sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+CLI_FLAGS = {"m": lambda v: ["-m", str(v)], "trans": lambda v: ["-" + v], "gcadjust": lambda v: [] if v else ["-NOGC"],
+             "cap": lambda v: ["-cap", str(v)], "merge": lambda v: [] if v else ["-nomerge"]}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("g", GOLD["depth_cases"], ids=lambda g: f"L{g['L']}-s{g['seed']}-{'-'.join(f'{k}{v}' for k, v in g['kw'].items()) or 'default'}")
+def test_cli_depth_file_matches_stored_reference_rows(g, cli, tmp_path):
+    """the CLI on a depth file of every stored case gives the rows the unmodified reference computed for it
+    (tests/golden/reference_vectors.json, tests/golden/make_golden.py)"""
+    from common import make_case
+    fa, d, _ = make_case(g["L"], g["seed"], stress=g["stress"])
+    assert _sha(d) + _sha(fa) == g["input_sha"], "synthetic input generator drifted"
+    fasta = str(tmp_path / "c.fa"); rd = str(tmp_path / "c.rd")
+    synth.write_fasta(fasta, "19", fa)
+    synth.write_depth_file_fast(rd, d)
+    flags = [f for k, v in g["kw"].items() for f in CLI_FLAGS[k](v)]
+    out = subprocess.run([cli, "rsi", "-d", rd, "-c", "19", "-f", fasta, "-np", "-o", str(tmp_path / "ours.txt")] + flags, capture_output=True, text=True)
+    assert out.returncode == 0, out.stderr
+    rows = [ln for ln in _table(str(tmp_path / "ours.txt")) if not ln.startswith("#")]
+    assert rows == g["rows"], out.stderr
+
+
+@pytest.mark.gpu
+def test_cli_bam_matches_stored_reference_table(cli, tmp_path):
+    """the stored BAM case (the reference CLI's `rsi -b ... -q 0 -Q 10 -np -s` table and the hash of its `-s` depth dump) through the
+    CLI on every decode route: per-GPU decoders from the index, one pass without it, host zlib"""
+    b = GOLD["bam_case"]
+    fa = synth.make_fasta(b["L"], b["seed"])
+    reads, _ = synth.make_reads(b["L"], b["seed"], fa, coverage=b["coverage"], n_events=b["n_events"], lens=tuple(b["lens"]))
+    assert _sha(reads["pos"]) + _sha(reads["qual"]) == b["reads_sha"], "synthetic read generator drifted"
+    bam = str(tmp_path / "t.bam"); fasta = str(tmp_path / "t.fa")
+    synth.write_fasta(fasta, "1", fa)
+    synth.write_bam(bam, [("1", b["L"])], {0: reads})
+    synth.write_bai(bam)
+    for extra, env in (([], {}), ([], {"RSICNV_NO_INDEX": "1"}), (["-hostdecode"], {})):
+        o = str(tmp_path / "ours.txt")
+        out = subprocess.run([cli, "rsi", "-b", bam, "-f", fasta, "-q", str(b["minq"]), "-Q", str(b["min_baseQ"]), "-np", "-s", "-o", o] + extra,
+                             capture_output=True, text=True, env=dict(os.environ, **env))
+        assert out.returncode == 0, (extra, env, out.stderr)
+        assert _table(o) == b["table"], (extra, env, out.stderr)
+        a = np.fromfile(o + ".1_rd", dtype=np.int64, sep=" ").reshape(-1, 2)
+        rd = np.zeros(b["L"], np.int32); rd[a[:, 0] - 1] = a[:, 1]
+        assert _sha(rd) == b["raw_depth_sha"], (extra, env)
+
+
+def _read_bai(path):
+    """per reference ({bin: [(beg, end), ...]}, linear index), and the trailing count of unplaced records (None if absent)"""
+    import struct
+    ix = open(path, "rb").read()
+    assert ix[:4] == b"BAI\x01"
+    o = 8; refs = []
+    for _ in range(struct.unpack_from("<i", ix, 4)[0]):
+        bins = {}
+        nbin = struct.unpack_from("<i", ix, o)[0]; o += 4
+        for _ in range(nbin):
+            b, nc = struct.unpack_from("<Ii", ix, o); o += 8
+            bins[b] = [struct.unpack_from("<QQ", ix, o + 16 * i) for i in range(nc)]; o += 16 * nc
+        ni = struct.unpack_from("<i", ix, o)[0]; o += 4
+        refs.append((bins, list(struct.unpack_from("<%dQ" % ni, ix, o)))); o += 8 * ni
+    return refs, (struct.unpack_from("<Q", ix, o)[0] if o + 8 <= len(ix) else None)
+
+
+def test_write_bai_indexes_every_record(tmp_path):
+    """synth.write_bai against the records of the file, walked here independently: every record lies in a chunk of its own bin,
+    the linear index never starts past a record of its window, the pseudo-bin holds the reference's file range and mapped /
+    unmapped counts, unplaced records are counted; where the reference's samtools is built, its index has the same content"""
+    import bisect
+    import struct
+    import zlib
+    r0, _ = synth.make_reads(300_000, 1, None, coverage=6, n_events=0, tid=0)
+    r2, _ = synth.make_reads(250_000, 2, None, coverage=5, n_events=0, tid=2, frac_indel=0.3)
+    bam = str(tmp_path / "t.bam")
+    synth.write_bam(bam, [("1", 300_000), ("2", 1000), ("3", 250_000)], {0: r0, 2: r2}, level=6, rich=5, unmapped_tail=11, block_size=20000)
+    synth.write_bai(bam)
+    refs, n_no_coor = _read_bai(bam + ".bai")
+    raw = open(bam, "rb").read(); dec = b""; fo, ds = [], []
+    off = 0
+    while off < len(raw):
+        xlen = struct.unpack_from("<H", raw, off + 10)[0]; bs = struct.unpack_from("<H", raw, off + 16)[0] + 1
+        fo.append(off); ds.append(len(dec)); dec += zlib.decompress(raw[off + 12 + xlen:off + bs - 8], -15); off += bs
+
+    def voff(x):
+        k = bisect.bisect_right(ds, x) - 1
+        return fo[k] << 16 | (x - ds[k])
+    lt = struct.unpack_from("<i", dec, 4)[0]; q = 12 + lt
+    for _ in range(struct.unpack_from("<i", dec, 8 + lt)[0]):
+        q += 8 + struct.unpack_from("<i", dec, q)[0]
+    recs = []
+    while q < len(dec):
+        bsz, tid, pos, bmn, fnc = struct.unpack_from("<iiiII", dec, q)
+        recs.append((tid, pos, bmn >> 16, fnc >> 16, voff(q), voff(q + 4 + bsz))); q += 4 + bsz
+    assert len(refs) == 3 and refs[1] == ({}, []) and n_no_coor == 11
+    for t, src in ((0, r0), (2, r2)):
+        mine = [r for r in recs if r[0] == t]
+        assert len(mine) == len(src["pos"])
+        bins, lin = refs[t]
+        for _, pos, b, flag, a, e in mine:
+            assert any(u <= a and e <= v for u, v in bins[b]), (t, pos, b)
+            assert lin[pos >> 14] <= a, (t, pos)
+        nmap = sum(1 for r in mine if not r[3] & 4)
+        assert bins[37450] == [(mine[0][4], mine[-1][5]), (nmap, len(mine) - nmap)]
+        assert min(u for b, ch in bins.items() if b != 37450 for u, _ in ch) == mine[0][4]
+    if have_ref():
+        ours = _read_bai(bam + ".bai")
+        subprocess.run([REF_BAMTOOL, "index", bam], check=True)
+        assert _read_bai(bam + ".bai") == ours
+
+
 def test_host_decoder_real_looking_records(cli, tmp_path):
     """the zlib reader on records with names, bases, optional fields and an unmapped tail"""
     r1, _ = synth.make_reads(120_000, 5, None, coverage=6, n_events=0, tid=0)
@@ -220,8 +337,7 @@ def test_cli_corrupt_bam_is_an_error_not_a_table(cli, tmp_path):
     bam = str(tmp_path / "t.bam"); fasta = str(tmp_path / "t.fa")
     synth.write_bam(bam, [("1", lens[0]), ("2", lens[1])], reads, level=1, random_seq=5)
     synth.write_fasta_multi(fasta, [("1", fas[0]), ("2", fas[1])])
-    if have_ref():
-        subprocess.run([REF_BAMTOOL, "index", bam], check=True)
+    synth.write_bai(bam)
     good = subprocess.run([cli, "rsi", "-b", bam, "-f", fasta, "-q", "0", "-Q", "10", "-np", "-o", str(tmp_path / "good.txt")], capture_output=True, text=True)
     assert good.returncode == 0, good.stderr
     rows = [ln for ln in _table(str(tmp_path / "good.txt")) if not ln.startswith("#")]

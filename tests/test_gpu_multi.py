@@ -14,7 +14,7 @@ import sys
 import numpy as np
 import pytest
 
-from bind import REF_BAMTOOL, REF_BIN, have_ref
+from bind import REF_BIN, have_ref
 from rsicnv_b200 import api, synth
 
 pytestmark = pytest.mark.gpu
@@ -73,8 +73,8 @@ def test_cli_two_gpus_equals_one(two_gpus, tmp_path):
     synth.write_fasta_multi(fasta, list(zip(names, fas)))
     common = ["rsi", "-b", bam, "-f", fasta, "-q", "0", "-Q", "10", "-np"]
     tables = {}
+    synth.write_bai(bam)
     if have_ref():
-        subprocess.run([REF_BAMTOOL, "index", bam], check=True)
         subprocess.run([REF_BIN] + common + ["-o", str(tmp_path / "ref.txt")], check=True, capture_output=True)
         tables["reference"] = _table(str(tmp_path / "ref.txt"))
     for key, extra, env in (("1gpu", ["-gpus", "1"], {}), ("2gpu_indexed", ["-gpus", "2"], {}), ("2gpu_one_pass", ["-gpus", "2"], {"RSICNV_NO_INDEX": "1"}),
@@ -164,8 +164,7 @@ def test_split_bam_contig_two_gpus_and_cli(two_gpus, gpu_lib, tmp_path):
     bam = str(tmp_path / "t.bam"); fasta = str(tmp_path / "t.fa"); rd = str(tmp_path / "t.rd")
     synth.write_bam(bam, [("7", L)], {0: reads}, level=1, random_seq=9)
     synth.write_fasta(fasta, "7", fa)
-    if have_ref():
-        subprocess.run([REF_BAMTOOL, "index", bam], check=True)
+    synth.write_bai(bam)
     depth, _ = synth.make_depth(L, 83, fa, n_events=6, lens=(3000, 8000, 20000))
     synth.write_depth_file_fast(rd, depth)
     for common in (["rsi", "-b", bam, "-f", fasta, "-q", "0", "-Q", "10", "-np"], ["rsi", "-d", rd, "-c", "7", "-f", fasta, "-np"]):
