@@ -228,6 +228,15 @@ int rsigpu_set_feed_limit(rsigpu_ctx* c, int64_t decoded_bytes);
 /* tuning / test hook: which inflate kernel rsigpu_bam_feed uses: 0 = by chunk size (default: a warp per BGZF block below
  * 28,000 blocks, a lane per block above), 1 = always a lane per block, 2 = always a warp per block; same bytes either way */
 int rsigpu_set_inflate_mode(rsigpu_ctx* c, int mode);
+/* on != 0: rsigpu_bam_feed and rsigpu_bam_feed_parts check the CRC32 of every BGZF block they decode (zlib's crc32 of the
+ * block's decoded bytes against the CRC in its gzip footer; a block with ISIZE 0 must carry CRC 0), on the GPU, after inflate.
+ * Default 0, like the reference's samtools-0.1.18 reader: without it, damage that leaves the deflate stream and the record
+ * cores valid (a changed quality byte or mate position, a bad footer) decodes without an error.  A mismatch fails the feed
+ * with RSIGPU_E_ARG before any run is reported or carried, naming the lowest failing block:
+ *   "bam_feed: CRC32 mismatch in BGZF block <k> of this feed (compressed offset <X> of the bytes passed)"
+ *   "bam_feed_parts: CRC32 mismatch in BGZF block <k> of part <j> (compressed offset <X> of that part)"
+ * A block whose deflate stream is corrupt is still reported as such; a CRC mismatch is reported before a corrupt record. */
+int rsigpu_set_bgzf_crc(rsigpu_ctx* c, int on);
 /* tuning hook: threads of the bin-level candidate kernel (multiple of 32, 32..1024) */
 int rsigpu_set_cand_threads(rsigpu_ctx* c, int threads);
 /* test hook: selected device-resident scalars of the last stage, as doubles; returns how many exist */

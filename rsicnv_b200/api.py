@@ -71,7 +71,7 @@ EXPORTS = ("rsigpu_default_params", "rsigpu_create", "rsigpu_destroy", "rsigpu_l
            "rsigpu_set_depth", "rsigpu_pileup_begin", "rsigpu_pileup_push", "rsigpu_pileup_end", "rsigpu_load_finish", "rsigpu_detectcnv",
            "rsigpu_sd_filters", "rsigpu_cnv_stat", "rsigpu_get_calls", "rsigpu_run", "rsigpu_get_chr_stats", "rsigpu_get_array",
            "rsigpu_format_row", "rsigpu_launch_count", "rsigpu_last_stage_ms", "rsigpu_set_profile", "rsigpu_get_profile",
-           "rsigpu_get_log", "rsigpu_reads_begin", "rsigpu_stat_calls", "rsigpu_bam_take_range", "rsigpu_split_range", "rsigpu_split_run", "rsigpu_split_p2p_bytes", "rsigpu_set_level0_mode", "rsigpu_set_feed_limit", "rsigpu_set_inflate_mode", "rsigpu_set_cand_threads", "rsigpu_debug_state", "rsigpu_pileup_commit", "rsigpu_bam_begin", "rsigpu_bam_feed", "rsigpu_bam_feed_parts", "rsigpu_bam_take",
+           "rsigpu_get_log", "rsigpu_reads_begin", "rsigpu_stat_calls", "rsigpu_bam_take_range", "rsigpu_split_range", "rsigpu_split_run", "rsigpu_split_p2p_bytes", "rsigpu_set_level0_mode", "rsigpu_set_feed_limit", "rsigpu_set_inflate_mode", "rsigpu_set_bgzf_crc", "rsigpu_set_cand_threads", "rsigpu_debug_state", "rsigpu_pileup_commit", "rsigpu_bam_begin", "rsigpu_bam_feed", "rsigpu_bam_feed_parts", "rsigpu_bam_take",
            "rsigpu_bam_end", "rsigpu_bam_run_field", "rsigpu_pinned_alloc", "rsigpu_pinned_free")
 
 _libs: dict[str, C.CDLL] = {}
@@ -176,6 +176,8 @@ class Context:
         mode = int(os.environ.get("RSIGPU_INFLATE_MODE", "0") or 0)      # test hook: force one of the two inflate kernels (rsigpu_set_inflate_mode)
         if mode:
             self.set_inflate_mode(mode)
+        if int(os.environ.get("RSIGPU_BGZF_CRC", "0") or 0):           # run any decode with the CRC32 check on (rsigpu_set_bgzf_crc)
+            self.set_bgzf_crc(True)
 
     def close(self):
         if getattr(self, "h", None):
@@ -418,6 +420,10 @@ class Context:
     def set_inflate_mode(self, mode: int):
         """0 = by chunk size, 1 = one lane per BGZF block, 2 = one warp per BGZF block"""
         self._ck(self.lib.rsigpu_set_inflate_mode(self.h, C.c_int(mode)))
+
+    def set_bgzf_crc(self, on: bool):
+        """check the CRC32 of every BGZF block bam_feed / bam_feed_parts decode (off by default, like the reference's reader)"""
+        self._ck(self.lib.rsigpu_set_bgzf_crc(self.h, C.c_int(1 if on else 0)))
 
     def set_feed_limit(self, decoded_bytes: int):
         """test hook: decoded bytes one bam_feed may produce"""

@@ -56,9 +56,9 @@ enum {
 enum { BAM_HEAD = 16 << 20 };      // room in front of the decoded blocks for the partial record carried from the previous chunk
 #define BAM_NONE (-1ll)
 #define BAM_TAIL 0x7fffffffffffffffll
-enum { BAM_ERR_INFLATE = 1, BAM_ERR_RECORD = 2, BAM_ERR_RUNS = 4 };
+enum { BAM_ERR_INFLATE = 1, BAM_ERR_RECORD = 2, BAM_ERR_RUNS = 4, BAM_ERR_CRC = 8 };
 
-struct BgzfBlock { u64 dst; u32 src, src_len, dst_len, pad_; };   // payload offset/length in the compressed chunk, offset/length in the decoded buffer
+struct BgzfBlock { u64 dst; u32 src, src_len, dst_len, crc; };   // payload offset/length in the compressed chunk, offset/length in the decoded buffer, footer CRC32
 
 struct BitIn {
   const u8* base; u32 pos, end;   // word-aligned base, next byte to load, one past the payload (both relative to base)

@@ -20,6 +20,7 @@
 
 #include "../../include/rsigpu.h"
 #include "k_bam.cuh"
+#include "k_crc32.cuh"
 
 using namespace rsigpu;
 
@@ -156,6 +157,7 @@ struct rsigpu_ctx {
   int b_nref = 0, b_tail_len = 0, b_rewalked = 0; bool b_active = false, b_first_feed = true;
   size_t b_umax = (size_t)5 << 30;   // decoded bytes one feed may produce (test hook: rsigpu_set_feed_limit)
   int inflate_mode = 0;              // 0 = by chunk size, 1 = one lane per BGZF block, 2 = one warp per BGZF block (rsigpu_set_inflate_mode)
+  bool bgzf_crc = false;             // check every block's CRC32 after inflate (rsigpu_set_bgzf_crc)
   // accounting
   long long h_cprof[16] = {};
   int64_t launches = 0;
@@ -263,6 +265,7 @@ int set_smem_attrs(int device) {
   // occupancy of these two is set by shared memory: ask for the largest shared-memory carve-out
   cudaFuncSetAttribute(k_rsi_scan_small, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
   cudaFuncSetAttribute(k_bgzf_inflate, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+  cudaFuncSetAttribute(k_bgzf_crc32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CRC_SMEM);
   return 0;
 }
 
@@ -566,9 +569,10 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
     if (off - base + bsize > (size_t)nbytes) break;
     const uint8_t* foot = h + bsize - 8;
     const size_t ulen = (size_t)foot[4] | ((size_t)foot[5] << 8) | ((size_t)foot[6] << 16) | ((size_t)foot[7] << 24);
+    const u32 crc = (u32)foot[0] | ((u32)foot[1] << 8) | ((u32)foot[2] << 16) | ((u32)foot[3] << 24);
     if (ulen > 65536) { c->fail("bam_feed: BGZF block larger than 64 KiB"); return RSIGPU_E_ARG; }
     if (utotal + ulen > U_MAX || off + bsize > C_MAX) break;
-    BgzfBlock B; B.src = (u32)(off + 12 + xlen); B.src_len = (u32)(bsize - 12 - xlen - 8); B.dst = (u64)BAM_HEAD + utotal; B.dst_len = (u32)ulen; B.pad_ = 0;
+    BgzfBlock B; B.src = (u32)(off + 12 + xlen); B.src_len = (u32)(bsize - 12 - xlen - 8); B.dst = (u64)BAM_HEAD + utotal; B.dst_len = (u32)ulen; B.crc = crc;
     blk.push_back(B);
     utotal += ulen; off += bsize;
     bound.push_back((i64)(BAM_HEAD + utotal));
@@ -603,6 +607,7 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
     CK(c->b_tabs.ensure(RSI_INFLATE_TAB_BYTES(nblk) / 2));
     KL(k_bgzf_inflate, (nblk + INF_NT - 1) / INF_NT, INF_NT, 0, c->b_comp.p, c->b_blk.p, nblk, c->b_U.p, c->b_tabs.p, err);
   }
+  if (c->bgzf_crc) KL(k_bgzf_crc32, grid_for(nblk, CRC_WARPS, c->n_sm), CRC_NT, CRC_SMEM, c->b_U.p, c->b_blk.p, nblk, err);
   BamChunk C; C.U = c->b_U.p; C.u_begin = c->b_first_feed ? (i64)BAM_HEAD + skip : (i64)BAM_HEAD - c->b_tail_len; C.u_end = (i64)(BAM_HEAD + utotal);
   C.bound = c->b_bound.p; C.nblk = nblk; C.n_ref = c->b_nref;
   BamChain H; H.first = c->b_first.p; H.endp = c->b_endp.p; H.tailp = c->b_tailp.p; H.cnt = c->b_cnt.p; H.ncig = c->b_ncig.p; H.nq = c->b_nq.p;
@@ -614,6 +619,16 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
   CK(cudaMemcpyAsync(he, err, 4 * 4, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
   if (he[1] & BAM_ERR_INFLATE) { c->fail("bam_feed: corrupt deflate stream in a BGZF block (code " + std::to_string(he[2]) + ")"); return RSIGPU_E_ARG; }
+  if (he[1] & BAM_ERR_CRC) {           // he[3] = nblk - (lowest failing block)
+    const int k = nblk - he[3];
+    int pj = 0; while (pj + 1 < nparts && part_blk[(size_t)pj + 1] <= k) ++pj;
+    // blocks of a part are contiguous: block k starts where block k - 1 of the same part ends
+    const size_t start = k == part_blk[(size_t)pj] ? part_off[(size_t)pj] : (size_t)blk[(size_t)k - 1].src + blk[(size_t)k - 1].src_len + 8;
+    if (multi) c->fail("bam_feed_parts: CRC32 mismatch in BGZF block " + std::to_string(k - part_blk[(size_t)pj]) + " of part " + std::to_string(pj) +
+                       " (compressed offset " + std::to_string(start - part_off[(size_t)pj]) + " of that part)");
+    else c->fail("bam_feed: CRC32 mismatch in BGZF block " + std::to_string(k) + " of this feed (compressed offset " + std::to_string(start) + " of the bytes passed)");
+    return RSIGPU_E_ARG;
+  }
   if (he[1] & BAM_ERR_RECORD) { c->fail("bam_feed: corrupt BAM record"); return RSIGPU_E_ARG; }
   const size_t n = (size_t)hi[0], ncg = (size_t)hi[1]; const i64 nq64 = hi[2];
   const i64 tail_start = hi[3];
@@ -1540,6 +1555,11 @@ int rsigpu_set_level0_mode(rsigpu_ctx* c, int mode) {
 int rsigpu_set_inflate_mode(rsigpu_ctx* c, int mode) {
   if (!c || mode < 0 || mode > 2) return RSIGPU_E_ARG;
   c->inflate_mode = mode;
+  return RSIGPU_OK;
+}
+int rsigpu_set_bgzf_crc(rsigpu_ctx* c, int on) {
+  if (!c) return RSIGPU_E_ARG;
+  c->bgzf_crc = on != 0;
   return RSIGPU_OK;
 }
 int rsigpu_set_feed_limit(rsigpu_ctx* c, int64_t decoded_bytes) {

@@ -37,7 +37,7 @@ namespace {
 
 struct Opt {
   std::string function = "rsi", rdfile, bamfile, reffile, cnvfile, outfile = "rsiout.txt", chr = "1-22XY";
-  bool saverd = false, hostdecode = false;
+  bool saverd = false, hostdecode = false, crc = false;
   int gpus = 1, threads = 8, split = 1;
   rsigpu_params P;
 };
@@ -48,7 +48,8 @@ int usage() {
           "Options:\n   -o  STR  outputfile [rsiout.txt]\n   -c  STR  chromosome [1-22XY]\n   -m  INT  bin size, odd [101]\n"
           "   -q  INT  minimum mapping quality [0]\n   -Q  INT  minimum base quality [13]\n   -cap FLT cap depth at FLT x median, <=1 off [4]\n"
           "   -NOGC    no GC adjustment\n   -MED | -NB | -ALL  transformation [NB]\n   -s       save raw depth to <out>.<chr>_rd (BAM input)\n"
-          "   -gpus INT  GPUs to shard contigs over [1]\n   -split INT  spread EVERY contig over INT GPUs instead (base ranges + halos, identical table) [1]\n   -hostdecode  inflate/parse the BAM on the host (zlib, -threads INT [8]) instead of on the GPU\n");
+          "   -gpus INT  GPUs to shard contigs over [1]\n   -split INT  spread EVERY contig over INT GPUs instead (base ranges + halos, identical table) [1]\n   -hostdecode  inflate/parse the BAM on the host (zlib, -threads INT [8]) instead of on the GPU\n"
+          "   -crc     check the CRC32 of every BGZF block the GPU decodes (the host decoder always does)\n");
   return 0;
 }
 
@@ -90,6 +91,7 @@ bool parse(int argc, char** argv, Opt* o) {
     if (k == "-split") { o->split = atoi(val(i).c_str()); two(); continue; }
     if (k == "-threads") { o->threads = atoi(val(i).c_str()); two(); continue; }
     if (k == "-hostdecode") { o->hostdecode = true; a[i] = ""; continue; }
+    if (k == "-crc") { o->crc = true; a[i] = ""; continue; }
   }
   bool bad = false;
   for (size_t i = 1; i < a.size(); ++i) if (!a[i].empty()) { fprintf(stderr, "unknown option %s\n", a[i].c_str()); bad = true; }
@@ -101,6 +103,13 @@ bool parse(int argc, char** argv, Opt* o) {
   if (!o->rdfile.empty() && (o->chr.empty() || o->chr == "1-22XY")) { fprintf(stderr, "readdepth file and chromosome must be specified together\n"); return false; }
   if (o->P.m % 2 != 1) { o->P.m += 1; fprintf(stderr, "m is changed to %d\n", o->P.m); }
   return true;
+}
+
+// a context that only decodes BAM bytes (rsigpu_bam_feed), with the CRC32 check of -crc
+int create_decoder(const Opt& o, int device, rsigpu_ctx** dec) {
+  const int rc = rsigpu_create(device, &o.P, dec);
+  if (rc) return rc;
+  return rsigpu_set_bgzf_crc(*dec, o.crc ? 1 : 0);
 }
 
 // read_fasta (readref.cpp:10-86): contig `chr` or "chr"+chr through the .fai index, newlines stripped
@@ -418,7 +427,7 @@ int bam_split_on_gpu(const Opt& o, std::vector<rsigpu_ctx*>& parts, std::vector<
   std::vector<BaiRef> bai;
   const bool indexed = !getenv("RSICNV_NO_INDEX") && read_bai(o.bamfile, h.name.size(), &bai);
   rsigpu_ctx* dec = nullptr;
-  if (rsigpu_create(0, &o.P, &dec)) { fprintf(stderr, "cannot create the decoder context\n"); return 2; }
+  if (create_decoder(o, 0, &dec)) { fprintf(stderr, "cannot create the decoder context\n"); return 2; }
   DecodeTiming tm; int failed = 0;
   std::vector<int32_t> pbeg((size_t)np), pend((size_t)np); int32_t halo = 0;
   auto start = [&](int tid) -> bool {      // FASTA to every part, read staging opened
@@ -525,7 +534,7 @@ int bam_on_gpu(const Opt& o, const std::vector<std::vector<rsigpu_ctx*>>& ctx, s
         for (int t = 0; t < n_ref; ++t) if (gpu_of[(size_t)t] == g) tids.push_back(t);
         if (tids.empty()) return;
         rsigpu_ctx* dec = nullptr;
-        if (rsigpu_create(g, &o.P, &dec)) { for (int t : tids) fail_contig(t, "cannot create the decoder context"); return; }
+        if (create_decoder(o, g, &dec)) { for (int t : tids) fail_contig(t, "cannot create the decoder context"); return; }
         FastaPrefetch fp(o.reffile);
         fp.request(h.name[(size_t)tids[0]]);
         std::thread fin[2];
@@ -563,7 +572,7 @@ int bam_on_gpu(const Opt& o, const std::vector<std::vector<rsigpu_ctx*>>& ctx, s
     for (auto& l : lanes) l.join();
   } else {
     rsigpu_ctx* dec = nullptr;
-    if (rsigpu_create(0, &o.P, &dec)) { fprintf(stderr, "cannot create the decoder context\n"); return 2; }
+    if (create_decoder(o, 0, &dec)) { fprintf(stderr, "cannot create the decoder context\n"); return 2; }
     if (rsigpu_bam_begin(dec, (int32_t)n_ref)) { fprintf(stderr, "%s\n", rsigpu_last_error(dec)); return 2; }
     std::vector<std::vector<std::thread>> fin((size_t)ng);
     for (int g = 0; g < ng; ++g) fin[(size_t)g].resize(ctx[(size_t)g].size());
@@ -655,7 +664,7 @@ int do_stat(const Opt& o, rsigpu_ctx* c) {
   std::vector<char> wanted((size_t)n_ref, 0);
   for (const rsigpu_cnv& x : list) if (x.tid >= 0) wanted[(size_t)x.tid] = 1;
   rsigpu_ctx* dec = nullptr;
-  if (rsigpu_create(0, &o.P, &dec)) { fprintf(stderr, "cannot create the decoder context\n"); return 2; }
+  if (create_decoder(o, 0, &dec)) { fprintf(stderr, "cannot create the decoder context\n"); return 2; }
   std::vector<BaiRef> bai;
   const bool indexed = !getenv("RSICNV_NO_INDEX") && read_bai(o.bamfile, h.name.size(), &bai);
   DecodeTiming tm;
