@@ -160,6 +160,28 @@ int rsigpu_bam_end(rsigpu_ctx* c);
 /* one decoded field of a run copied to the host (parity tests): 0 pos, 1 mpos, 2 isize, 3 mtid (int32), 4 flag (uint16),
  * 5 mapq (uint8), 6 cigar_off (uint32, n+1, rebased to 0), 7 cigar (uint32), 8 qual_off (uint64, n+1, rebased), 9 qual (uint8) */
 int rsigpu_bam_run_field(rsigpu_ctx* c, int32_t run, int32_t field, void* out, int64_t cap_bytes, int64_t* nbytes);
+/* The BAI index of the file (SAM spec 5.2, byte for byte what samtools-0.1.18's bam_index_build writes) built on the GPU from
+ * the records rsigpu_bam_feed decodes anyway: no second pass over the file.
+ *   index_begin(file_offset)   after rsigpu_bam_begin, before the first feed.  file_offset = offset in the FILE of the first byte
+ *                              the first feed receives (the BGZF block that holds the first record).  Every later feed must
+ *                              continue the file where the previous one's *consumed ended; the offsets of the index follow.
+ *   feeds as usual, then rsigpu_bam_end
+ *   index_get(out, cap, &n)    the serialized .bai, valid after a successful rsigpu_bam_end; out == NULL: only *nbytes.
+ * While indexing, a feed additionally fails
+ *   with RSIGPU_E_ARG    "bam_index: records not sorted: record <k> of this feed (tid <t>, pos <p>) follows tid <t'>, pos <p'>"
+ *                        (the lowest such record: refIDs must not decrease -- unplaced records, refID -1, come last -- and
+ *                        positions must not decrease within a reference; reported after inflate, CRC and record errors)
+ *   with RSIGPU_E_RANGE  "bam_index: record <k> of this feed (tid <t>, pos <p>) ends past 2^29, beyond what a BAI index can address"
+ * and rsigpu_bam_feed_parts fails with RSIGPU_E_ARG (its parts are not one contiguous file):
+ *   "bam_feed_parts: not available while a BAM index is built (rsigpu_bam_index_begin): its parts are not one contiguous file"
+ * index_begin fails with RSIGPU_E_ARG after the first feed or without rsigpu_bam_begin:
+ *   "bam_index_begin: call it after rsigpu_bam_begin and before the first feed, with the file offset of the first byte fed"
+ * index_get fails with RSIGPU_E_ARG when any feed or rsigpu_bam_end failed, or indexing was never begun:
+ *   "bam_index_get: no index: rsigpu_bam_index_begin, feeds of the whole file and rsigpu_bam_end must all succeed first"
+ * and with RSIGPU_E_CAPACITY when cap < *nbytes: "bam_index_get: the buffer is smaller than the index".
+ * Without index_begin nothing of this runs: no extra launch, no extra copy. */
+int rsigpu_bam_index_begin(rsigpu_ctx* c, int64_t file_offset);
+int rsigpu_bam_index_get(rsigpu_ctx* c, uint8_t* out, int64_t cap, int64_t* nbytes);
 int rsigpu_pinned_alloc(size_t nbytes, void** out);
 void rsigpu_pinned_free(void* p);
 

@@ -72,7 +72,7 @@ EXPORTS = ("rsigpu_default_params", "rsigpu_create", "rsigpu_destroy", "rsigpu_l
            "rsigpu_sd_filters", "rsigpu_cnv_stat", "rsigpu_get_calls", "rsigpu_run", "rsigpu_get_chr_stats", "rsigpu_get_array",
            "rsigpu_format_row", "rsigpu_launch_count", "rsigpu_last_stage_ms", "rsigpu_set_profile", "rsigpu_get_profile",
            "rsigpu_get_log", "rsigpu_reads_begin", "rsigpu_stat_calls", "rsigpu_bam_take_range", "rsigpu_split_range", "rsigpu_split_run", "rsigpu_split_p2p_bytes", "rsigpu_set_level0_mode", "rsigpu_set_feed_limit", "rsigpu_set_inflate_mode", "rsigpu_set_bgzf_crc", "rsigpu_set_cand_threads", "rsigpu_debug_state", "rsigpu_pileup_commit", "rsigpu_bam_begin", "rsigpu_bam_feed", "rsigpu_bam_feed_parts", "rsigpu_bam_take",
-           "rsigpu_bam_end", "rsigpu_bam_run_field", "rsigpu_pinned_alloc", "rsigpu_pinned_free")
+           "rsigpu_bam_end", "rsigpu_bam_run_field", "rsigpu_bam_index_begin", "rsigpu_bam_index_get", "rsigpu_pinned_alloc", "rsigpu_pinned_free")
 
 _libs: dict[str, C.CDLL] = {}
 
@@ -287,6 +287,19 @@ class Context:
 
     def bam_end(self):
         self._ck(self.lib.rsigpu_bam_end(self.h))
+
+    def bam_index_begin(self, file_offset: int):
+        """build the file's .bai while it is decoded (rsigpu_bam_index_begin): call after bam_begin, before the first feed;
+        file_offset = offset in the file of the first byte fed, and every feed must continue where the last one's consumed ended"""
+        self._ck(self.lib.rsigpu_bam_index_begin(self.h, C.c_int64(file_offset)))
+
+    def bam_index(self) -> bytes:
+        """the .bai bytes after a successful bam_end (rsigpu_bam_index_get)"""
+        nb = C.c_int64(0)
+        self._ck(self.lib.rsigpu_bam_index_get(self.h, None, C.c_int64(0), C.byref(nb)))
+        buf = (C.c_uint8 * max(nb.value, 1))()
+        self._ck(self.lib.rsigpu_bam_index_get(self.h, buf, C.c_int64(nb.value), C.byref(nb)))
+        return bytes(buf[:nb.value])
 
     _BAM_FIELDS = (("pos", np.int32), ("mpos", np.int32), ("isize", np.int32), ("mtid", np.int32), ("flag", np.uint16), ("mapq", np.uint8),
                    ("cigar_off", np.uint32), ("cigar", np.uint32), ("qual_off", np.uint64), ("qual", np.uint8))

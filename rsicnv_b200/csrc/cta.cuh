@@ -132,6 +132,27 @@ struct Cta {
     *total = all;
     return before + base + inc - v;
   }
+  // exclusive scan under any associative, commutative op with identity `id` (one block: nctas == 1); *total to every thread
+  template <class T, class Op>
+  RSI_DEV T scan_excl_op(T v, Op op, T id, T* total) const {
+    const int t = lt(), warp = t >> 5, lane = t & 31, nw = (ln() + 31) >> 5;
+    T inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      T up = shfl_up_any(inc, o);
+      if (lane >= o) inc = op(inc, up);
+    }
+    T ex = shfl_up_any(inc, 1);
+    if (lane == 0) ex = id;
+    T* slots = reinterpret_cast<T*>(red);
+    __syncthreads();
+    if (lane == 31) slots[warp] = inc;
+    __syncthreads();
+    T base = id, tot = id;
+    for (int w = 0; w < nw; ++w) { T sv = slots[w]; if (w < warp) base = op(base, sv); tot = op(tot, sv); }
+    *total = tot;
+    return op(base, ex);
+  }
   // out-of-line forms for the candidate kernels: their time is instruction FETCH (k_cand_a: 300 KB of SASS that one block runs
   // through once), and ~100 inlined copies of these two are a quarter of it.  The streaming kernels keep the inline forms: a
   // call inside their tile loops costs far more than it saves (k_pileup_tile 0.49 -> 1.48 ms when tried).

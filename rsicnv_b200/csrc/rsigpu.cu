@@ -21,6 +21,7 @@
 #include "../../include/rsigpu.h"
 #include "k_bam.cuh"
 #include "k_crc32.cuh"
+#include "k_bam_index.cuh"
 
 using namespace rsigpu;
 
@@ -158,6 +159,16 @@ struct rsigpu_ctx {
   size_t b_umax = (size_t)5 << 30;   // decoded bytes one feed may produce (test hook: rsigpu_set_feed_limit)
   int inflate_mode = 0;              // 0 = by chunk size, 1 = one lane per BGZF block, 2 = one warp per BGZF block (rsigpu_set_inflate_mode)
   bool bgzf_crc = false;             // check every block's CRC32 after inflate (rsigpu_set_bgzf_crc)
+  // BAI index built from the decoded records (k_bam_index.cuh, rsigpu_bam_index_begin / _get)
+  struct IxChunk { u32 bin; u64 u, v; };
+  struct IxRef { std::vector<IxChunk> ch; u64 n_map = 0, n_unmap = 0; std::vector<u64> lin; };
+  bool ix_on = false, ix_failed = false, ix_ready = false, ix_has_prev = false;
+  int64_t ix_off = 0;                // file offset of the next feed's first byte
+  u64 ix_carry_voff = 0, ix_end_voff = 0, ix_prev_key = 0, ix_no_coor = 0;
+  int ix_prev_tid = 0, ix_prev_pos = 0; u32 ix_prev_bin = 0;
+  IxChunk ix_pend{}; int ix_pend_tid = -1; bool ix_pend_on = false;   // the last run seen: its end is the next run's begin
+  std::vector<IxRef> ix_ref; std::vector<uint8_t> ix_out;
+  DevBuf<u64> x_beg, x_key, x_cnt, x_tkey; DevBuf<u32> x_meta; DevBuf<int> x_tstart, x_tunmap; DevBuf<BixChunk> x_chunk; DevBuf<BixLin> x_lin;
   // accounting
   long long h_cprof[16] = {};
   int64_t launches = 0;
@@ -402,6 +413,7 @@ void rsigpu_destroy(rsigpu_ctx* c) {
   c->b_bound.release(); c->b_first.release(); c->b_endp.release(); c->b_tailp.release(); c->b_cnt.release(); c->b_ncig.release(); c->b_in.release(); c->b_rbase.release(); c->b_cbase.release();
   c->b_info.release(); c->b_runstart.release(); c->b_rec.release(); c->b_tid.release(); c->b_pos.release(); c->b_mpos.release(); c->b_isize.release(); c->b_mtid.release();
   c->b_nq.release(); c->b_qbase.release(); c->b_runinfo.release();
+  c->x_beg.release(); c->x_key.release(); c->x_cnt.release(); c->x_tkey.release(); c->x_meta.release(); c->x_tstart.release(); c->x_tunmap.release(); c->x_chunk.release(); c->x_lin.release();
   if (c->d_st) cudaFree(c->d_st);
   if (c->h_st) cudaFreeHost(c->h_st);
   if (c->h_lut) cudaFreeHost(c->h_lut);
@@ -528,6 +540,63 @@ int rsigpu_pileup_push(rsigpu_ctx* c, const rsigpu_read_batch* b) {
 int rsigpu_bam_begin(rsigpu_ctx* c, int32_t n_ref) {
   if (!c || n_ref < 1) return RSIGPU_E_ARG;
   c->b_nref = n_ref; c->b_tail_len = 0; c->b_active = true; c->b_first_feed = true; c->b_runs.clear(); c->b_rewalked = 0;
+  c->ix_on = false; c->ix_failed = false; c->ix_ready = false; c->ix_out.clear(); c->ix_ref.clear();
+  return RSIGPU_OK;
+}
+
+int rsigpu_bam_index_begin(rsigpu_ctx* c, int64_t file_offset) {
+  if (!c) return RSIGPU_E_ARG;
+  if (!c->b_active || !c->b_first_feed || file_offset < 0) { c->fail("bam_index_begin: call it after rsigpu_bam_begin and before the first feed, with the file offset of the first byte fed"); return RSIGPU_E_ARG; }
+  c->ix_on = true; c->ix_failed = false; c->ix_ready = false; c->ix_has_prev = false; c->ix_off = file_offset;
+  c->ix_carry_voff = 0; c->ix_end_voff = 0; c->ix_prev_key = 0; c->ix_no_coor = 0; c->ix_pend_on = false; c->ix_pend_tid = -1;
+  c->ix_out.clear(); c->ix_ref.assign((size_t)c->b_nref, rsigpu_ctx::IxRef());
+  return RSIGPU_OK;
+}
+
+// samtools-0.1.18's bam_index_save layout: per reference the bins in ascending order with their chunks (merge_chunks: a chunk
+// whose begin lies in the BGZF block where the previous chunk of its bin ends is joined to it), the pseudo-bin 37450 (file
+// range of the reference's records, mapped / unmapped counts), the 16 kbp linear index with uncovered windows taking the
+// previous window's offset; the count of unplaced records last, when there are any
+static void ix_serialize(rsigpu_ctx* c) {
+  std::vector<uint8_t>& o = c->ix_out;
+  o.clear();
+  auto put32 = [&](u32 v) { for (int k = 0; k < 4; ++k) o.push_back((uint8_t)(v >> (8 * k))); };
+  auto put64 = [&](u64 v) { for (int k = 0; k < 8; ++k) o.push_back((uint8_t)(v >> (8 * k))); };
+  o.push_back('B'); o.push_back('A'); o.push_back('I'); o.push_back(1);
+  put32((u32)c->ix_ref.size());
+  for (rsigpu_ctx::IxRef& R : c->ix_ref) {
+    if (R.ch.empty()) { put32(0); put32(0); continue; }
+    const u64 first = R.ch.front().u, last = R.ch.back().v;
+    std::stable_sort(R.ch.begin(), R.ch.end(), [](const rsigpu_ctx::IxChunk& a, const rsigpu_ctx::IxChunk& b) { return a.bin < b.bin; });
+    std::vector<rsigpu_ctx::IxChunk> m;
+    m.reserve(R.ch.size());
+    int nbin = 1;
+    for (const rsigpu_ctx::IxChunk& x : R.ch) {
+      if (!m.empty() && m.back().bin == x.bin && m.back().v >> 16 == x.u >> 16) m.back().v = x.v;
+      else { nbin += m.empty() || m.back().bin != x.bin; m.push_back(x); }
+    }
+    put32((u32)nbin);
+    for (size_t i = 0; i < m.size();) {
+      size_t j = i;
+      while (j < m.size() && m[j].bin == m[i].bin) ++j;
+      put32(m[i].bin); put32((u32)(j - i));
+      for (; i < j; ++i) { put64(m[i].u); put64(m[i].v); }
+    }
+    put32(37450u); put32(2); put64(first); put64(last); put64(R.n_map); put64(R.n_unmap);
+    for (size_t w = 1; w < R.lin.size(); ++w) if (!R.lin[w]) R.lin[w] = R.lin[w - 1];
+    put32((u32)R.lin.size());
+    for (u64 v : R.lin) put64(v);
+  }
+  if (c->ix_no_coor) put64(c->ix_no_coor);
+}
+
+int rsigpu_bam_index_get(rsigpu_ctx* c, uint8_t* out, int64_t cap, int64_t* nbytes) {
+  if (!c || !nbytes) return RSIGPU_E_ARG;
+  if (!c->ix_ready) { c->fail("bam_index_get: no index: rsigpu_bam_index_begin, feeds of the whole file and rsigpu_bam_end must all succeed first"); return RSIGPU_E_ARG; }
+  *nbytes = (int64_t)c->ix_out.size();
+  if (!out) return RSIGPU_OK;
+  if (cap < *nbytes) { c->fail("bam_index_get: the buffer is smaller than the index"); return RSIGPU_E_CAPACITY; }
+  memcpy(out, c->ix_out.data(), c->ix_out.size());
   return RSIGPU_OK;
 }
 
@@ -634,6 +703,8 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
   const i64 tail_start = hi[3];
   c->b_rewalked += (int)hi[4];
   c->b_first_feed = false;
+  u64 xc[BIX_C_N] = {};
+  std::vector<BixChunk> xchunk; std::vector<BixLin> xlin;
   if (n) {
     CK(c->b_rec.ensure(n)); CK(c->b_tid.ensure(n)); CK(c->b_pos.ensure(n)); CK(c->b_mpos.ensure(n)); CK(c->b_isize.ensure(n)); CK(c->b_mtid.ensure(n));
     CK(c->b_flag.ensure(n)); CK(c->b_mapq.ensure(n)); CK(c->b_cigoff.ensure(n + 1)); CK(c->b_qoff.ensure(n + 1)); CK(c->b_cig.ensure(ncg + 1)); CK(c->b_qual.ensure((size_t)nq64 + 16));
@@ -643,6 +714,22 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
     KL(k_bam_fields, (nblk + 127) / 128, 128, 0, C, H, c->b_rbase.p, c->b_cbase.p, c->b_qbase.p, info, S);
     KL(k_bam_payload, c->n_sm * 8, 256, 0, c->b_U.p, info, S);
     KL(k_bam_runs, grid_for((int)std::min<size_t>(n, 1u << 30), 1024, c->n_sm * 8), 256, 0, c->b_tid.p, info, c->b_runstart.p, (int)LIST_CAP, err);
+    if (c->ix_on) {          // the BAI index's share of this feed (k_bam_index.cuh); its counts travel with the error copy below
+      const int ntile = (int)((n + BIX_NT - 1) / BIX_NT);
+      CK(c->x_beg.ensure(n)); CK(c->x_key.ensure(n)); CK(c->x_meta.ensure(n)); CK(c->x_chunk.ensure(n)); CK(c->x_lin.ensure(n));
+      CK(c->x_tstart.ensure((size_t)ntile)); CK(c->x_tunmap.ensure((size_t)ntile)); CK(c->x_tkey.ensure((size_t)ntile)); CK(c->x_cnt.ensure(BIX_C_N));
+      CK(cudaMemsetAsync(c->x_cnt.p, 0, BIX_C_N * 8, c->stream));
+      BixFeed F;
+      F.U = c->b_U.p; F.bound = c->b_bound.p; F.blk = c->b_blk.p; F.nblk = nblk; F.base = (i64)c->ix_off; F.carry_voff = c->ix_carry_voff; F.n = (int)n;
+      F.rec = c->b_rec.p; F.tid = c->b_tid.p; F.pos = c->b_pos.p; F.flag = c->b_flag.p; F.cigar_off = c->b_cigoff.p; F.cigar = c->b_cig.p;
+      F.has_prev = c->ix_has_prev; F.prev_tid = c->ix_prev_tid; F.prev_pos = c->ix_prev_pos; F.prev_bin = c->ix_prev_bin; F.prev_key = c->ix_prev_key;
+      F.beg = c->x_beg.p; F.key = c->x_key.p; F.meta = c->x_meta.p; F.t_start = c->x_tstart.p; F.t_unmap = c->x_tunmap.p; F.t_key = c->x_tkey.p;
+      F.chunk = c->x_chunk.p; F.lin = c->x_lin.p; F.cnt = c->x_cnt.p;
+      KL(k_bam_index_rec, ntile, BIX_NT, 0, F);
+      KL(k_bam_index_scan, 1, BIX_SCAN_NT, 0, F, ntile);
+      KL(k_bam_index_emit, ntile, BIX_NT, 0, F);
+      CK(cudaMemcpyAsync(xc, c->x_cnt.p, BIX_C_N * 8, cudaMemcpyDeviceToHost, c->stream));
+    }
     std::vector<int> part_rec;           // first record of every part (each part starts a run whatever its refID)
     if (multi) {
       part_rec.resize((size_t)nparts);
@@ -650,6 +737,30 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
     }
     CK(cudaMemcpyAsync(he, err, 4 * 4, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
+    if (c->ix_on && xc[BIX_C_UNSORTED]) {
+      const i64 k = (i64)n - (i64)xc[BIX_C_UNSORTED];
+      int t[2] = {c->ix_prev_tid, 0}, q[2] = {c->ix_prev_pos, 0};
+      if (k > 0) { CK(cudaMemcpyAsync(t, c->b_tid.p + k - 1, 8, cudaMemcpyDeviceToHost, c->stream)); CK(cudaMemcpyAsync(q, c->b_pos.p + k - 1, 8, cudaMemcpyDeviceToHost, c->stream)); }
+      else { CK(cudaMemcpyAsync(t + 1, c->b_tid.p, 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaMemcpyAsync(q + 1, c->b_pos.p, 4, cudaMemcpyDeviceToHost, c->stream)); }
+      CK(cudaStreamSynchronize(c->stream));
+      c->fail("bam_index: records not sorted: record " + std::to_string(k) + " of this feed (tid " + std::to_string(t[1]) + ", pos " + std::to_string(q[1]) +
+              ") follows tid " + std::to_string(t[0]) + ", pos " + std::to_string(q[0]));
+      return RSIGPU_E_ARG;
+    }
+    if (c->ix_on && xc[BIX_C_RANGE]) {
+      const i64 k = (i64)n - (i64)xc[BIX_C_RANGE];
+      int t = 0, q = 0;
+      CK(cudaMemcpyAsync(&t, c->b_tid.p + k, 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaMemcpyAsync(&q, c->b_pos.p + k, 4, cudaMemcpyDeviceToHost, c->stream));
+      CK(cudaStreamSynchronize(c->stream));
+      c->fail("bam_index: record " + std::to_string(k) + " of this feed (tid " + std::to_string(t) + ", pos " + std::to_string(q) +
+              ") ends past 2^29, beyond what a BAI index can address");
+      return RSIGPU_E_RANGE;
+    }
+    if (c->ix_on) {        // copied with the run starts below
+      xchunk.resize((size_t)xc[BIX_C_CHUNKS]); xlin.resize((size_t)xc[BIX_C_LIN]);
+      if (!xchunk.empty()) CK(cudaMemcpyAsync(xchunk.data(), c->x_chunk.p, xchunk.size() * sizeof(BixChunk), cudaMemcpyDeviceToHost, c->stream));
+      if (!xlin.empty()) CK(cudaMemcpyAsync(xlin.data(), c->x_lin.p, xlin.size() * sizeof(BixLin), cudaMemcpyDeviceToHost, c->stream));
+    }
     if (he[1] & BAM_ERR_RUNS) { c->fail("bam_feed: more than 65536 refID runs in one chunk (the BAM is not coordinate-sorted)"); return RSIGPU_E_RANGE; }
     int nr = he[0];
     std::vector<int> rs((size_t)nr);
@@ -683,6 +794,34 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
     CK(cudaStreamSynchronize(c->stream));
   }
   c->b_tail_len = tail_len > 0 ? (int)tail_len : 0;
+  if (c->ix_on) {
+    // voffset of decoded position x: the last block that starts at or before it
+    auto voff_at = [&](i64 x) {
+      const int k = (int)(std::upper_bound(bound.begin(), bound.begin() + nblk, x) - bound.begin()) - 1;
+      const u64 co = (u64)c->ix_off + (k ? (u64)blk[(size_t)k - 1].src + blk[(size_t)k - 1].src_len + 8 : 0ull);
+      return (co << 16) | (u64)(x - bound[(size_t)k]);
+    };
+    for (size_t i = 0; i < xchunk.size(); ++i) {
+      const BixChunk& h = xchunk[i];
+      if (c->ix_pend_on && c->ix_pend_tid >= 0) { c->ix_pend.v = h.u; c->ix_ref[(size_t)c->ix_pend_tid].ch.push_back(c->ix_pend); }
+      c->ix_pend.bin = h.bin; c->ix_pend.u = h.u; c->ix_pend.v = 0; c->ix_pend_tid = h.tid; c->ix_pend_on = true;
+      const i64 nrec = (i + 1 < xchunk.size() ? (i64)xchunk[i + 1].rec : (i64)n) - h.rec;
+      const i64 nun = (i + 1 < xchunk.size() ? (i64)xchunk[i + 1].unmap : (i64)xc[BIX_C_UNMAP]) - h.unmap;
+      if (h.tid >= 0) { c->ix_ref[(size_t)h.tid].n_unmap += (u64)nun; c->ix_ref[(size_t)h.tid].n_map += (u64)(nrec - nun); }
+      else c->ix_no_coor += (u64)nrec;
+    }
+    for (const BixLin& L : xlin) {
+      std::vector<u64>& lin = c->ix_ref[(size_t)L.tid].lin;
+      if (lin.size() < (size_t)L.w1 + 1) lin.resize((size_t)L.w1 + 1, 0);
+      for (int w = L.w0; w <= L.w1; ++w) lin[(size_t)w] = L.voff;
+    }
+    if (n) { c->ix_has_prev = true; c->ix_prev_tid = (int)(u32)xc[BIX_C_LAST_TID]; c->ix_prev_pos = (int)(u32)xc[BIX_C_LAST_POS]; c->ix_prev_bin = (u32)xc[BIX_C_LAST_BIN]; c->ix_prev_key = xc[BIX_C_MAXKEY]; }
+    if (tail_len > 0) c->ix_carry_voff = voff_at(tail_start);
+    // where the stream stops if this is the last feed: an empty block at the end (the EOF marker) is that place, else the byte after the chunk
+    const i64 u_end = (i64)(BAM_HEAD + utotal);
+    c->ix_end_voff = bound[(size_t)nblk - 1] == u_end ? voff_at(u_end) : (u64)(c->ix_off + (int64_t)off) << 16;
+    c->ix_off += (int64_t)off;
+  }
   TRACE(c, "feed: end");
   if (consumed) *consumed = (int64_t)off;
   *n_runs = (int32_t)c->b_runs.size();
@@ -693,10 +832,13 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
 int rsigpu_bam_feed(rsigpu_ctx* c, const uint8_t* bgzf, int64_t nbytes, int64_t skip, int64_t* consumed, rsigpu_bam_run* runs, int32_t cap, int32_t* n_runs) {
   if (!bgzf || !consumed) return RSIGPU_E_ARG;
   const uint8_t* p[1] = {bgzf}; const int64_t n[1] = {nbytes};
-  return bam_feed_impl(c, 1, p, n, skip, consumed, runs, cap, n_runs);
+  const int rc = bam_feed_impl(c, 1, p, n, skip, consumed, runs, cap, n_runs);
+  if (rc != RSIGPU_OK && c) c->ix_failed = true;     // an index missing this feed's records would be wrong: rsigpu_bam_index_get refuses
+  return rc;
 }
 int rsigpu_bam_feed_parts(rsigpu_ctx* c, int32_t n_parts, const uint8_t* const* parts, const int64_t* nbytes, rsigpu_bam_run* runs, int32_t cap, int32_t* n_runs) {
   if (n_parts < 1) return RSIGPU_E_ARG;
+  if (c && c->ix_on) { c->ix_failed = true; c->fail("bam_feed_parts: not available while a BAM index is built (rsigpu_bam_index_begin): its parts are not one contiguous file"); return RSIGPU_E_ARG; }
   if (n_parts == 1) { int64_t consumed = 0; const int rc = bam_feed_impl(c, 1, parts, nbytes, 0, &consumed, runs, cap, n_runs); if (rc == RSIGPU_OK && consumed != nbytes[0]) { c->fail("bam_feed_parts: a part is not a whole number of BGZF blocks"); return RSIGPU_E_RANGE; } return rc; }
   return bam_feed_impl(c, n_parts, parts, nbytes, 0, nullptr, runs, cap, n_runs);
 }
@@ -747,6 +889,16 @@ int rsigpu_bam_end(rsigpu_ctx* c) {
   if (!c) return RSIGPU_E_ARG;
   const bool cut = c->b_active && c->b_tail_len > 0;
   c->b_active = false; c->b_runs.clear(); c->b_tail_len = 0;
+  if (c->ix_on) {
+    c->ix_on = false;
+    if (!cut && !c->ix_failed) {
+      if (c->ix_pend_on && c->ix_pend_tid >= 0) { c->ix_pend.v = c->ix_end_voff; c->ix_ref[(size_t)c->ix_pend_tid].ch.push_back(c->ix_pend); }
+      c->ix_pend_on = false;
+      ix_serialize(c);
+      c->ix_ref.clear();
+      c->ix_ready = true;
+    }
+  }
   if (cut) { c->fail("bam_end: the BAM stream stops inside an alignment record"); return RSIGPU_E_ARG; }
   return RSIGPU_OK;
 }

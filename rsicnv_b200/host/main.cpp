@@ -10,6 +10,8 @@
 //
 // Extra sub-command for the tests (no GPU needed):  rsicnv decode -b in.bam -c CHR -o prefix
 //   writes the decoded structure-of-arrays of one contig as raw little-endian files prefix.<field>.
+// `rsicnv index -b in.bam [-o out.bai]` writes the BAI index (default in.bam.bai, samtools' name), built on GPU 0 while it
+//   decodes the file in one pass (rsigpu_bam_index_begin): what `rsi` and `stat` read to decode every contig from its own offset.
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -37,7 +39,7 @@ namespace {
 
 struct Opt {
   std::string function = "rsi", rdfile, bamfile, reffile, cnvfile, outfile = "rsiout.txt", chr = "1-22XY";
-  bool saverd = false, hostdecode = false, crc = false;
+  bool saverd = false, hostdecode = false, crc = false, out_set = false;
   int gpus = 1, threads = 8, split = 1;
   rsigpu_params P;
 };
@@ -45,6 +47,7 @@ struct Opt {
 int usage() {
   fprintf(stderr,
           "Usage:\n  rsicnv rsi -f REF -b BAM [options]\n  rsicnv rsi -f REF -d RDFILE -c CHR [options]\n"
+          "  rsicnv index -b BAM [-o OUT] [-crc]   write the BAI index (default BAM.bai), built on the GPU\n"
           "Options:\n   -o  STR  outputfile [rsiout.txt]\n   -c  STR  chromosome [1-22XY]\n   -m  INT  bin size, odd [101]\n"
           "   -q  INT  minimum mapping quality [0]\n   -Q  INT  minimum base quality [13]\n   -cap FLT cap depth at FLT x median, <=1 off [4]\n"
           "   -NOGC    no GC adjustment\n   -MED | -NB | -ALL  transformation [NB]\n   -s       save raw depth to <out>.<chr>_rd (BAM input)\n"
@@ -59,7 +62,7 @@ bool parse(int argc, char** argv, Opt* o) {
   if (a.size() < 2) return false;
   if (a[1][0] != '-') {
     o->function = a[1]; a[1] = "";
-    if (o->function != "rsi" && o->function != "decode" && o->function != "stat") { fprintf(stderr, "no such function %s (this build implements `rsi` and `stat`)\n", o->function.c_str()); return false; }
+    if (o->function != "rsi" && o->function != "decode" && o->function != "stat" && o->function != "index") { fprintf(stderr, "no such function %s (this build implements `rsi`, `stat` and `index`)\n", o->function.c_str()); return false; }
   }
   auto val = [&](size_t i) { return i + 1 < a.size() ? a[i + 1] : std::string(); };
   for (size_t i = 1; i < a.size(); ++i) {
@@ -69,7 +72,7 @@ bool parse(int argc, char** argv, Opt* o) {
     if (k == "-b") { o->bamfile = val(i); two(); continue; }
     if (k == "-f") { o->reffile = val(i); two(); continue; }
     if (k == "-v") { o->cnvfile = val(i); two(); continue; }
-    if (k == "-o") { o->outfile = val(i); two(); continue; }
+    if (k == "-o") { o->outfile = val(i); o->out_set = true; two(); continue; }
     if (k == "-c") { o->chr = val(i); two(); continue; }
     if (k == "-s") { o->saverd = true; a[i] = ""; continue; }
     if (k == "-m") { o->P.m = atoi(val(i).c_str()); two(); continue; }
@@ -99,6 +102,7 @@ bool parse(int argc, char** argv, Opt* o) {
   if (o->rdfile.empty() && o->bamfile.empty()) { fprintf(stderr, "need input file \n"); return false; }
   if (o->reffile.empty() && o->function == "rsi") { fprintf(stderr, "need reference file \n"); return false; }
   if (o->function == "stat" && (o->bamfile.empty() || o->cnvfile.empty())) { fprintf(stderr, "stat needs -b BAM and -v CNVFILE\n"); return false; }
+  if (o->function == "index" && o->bamfile.empty()) { fprintf(stderr, "index needs -b BAM\n"); return false; }
   if (o->outfile == o->bamfile || o->outfile == o->rdfile) { fprintf(stderr, "output file is same as input file \n"); return false; }
   if (!o->rdfile.empty() && (o->chr.empty() || o->chr == "1-22XY")) { fprintf(stderr, "readdepth file and chromosome must be specified together\n"); return false; }
   if (o->P.m % 2 != 1) { o->P.m += 1; fprintf(stderr, "m is changed to %d\n", o->P.m); }
@@ -745,6 +749,40 @@ void write_log(const Opt& o, const std::string& command, const std::vector<Conti
   fclose(f);
 }
 
+// `rsicnv index`: the file streamed through one decoder on GPU 0 with indexing on, the same chunks as the one-pass route.  The
+// index goes to a temporary name first and is renamed into place only when every feed succeeded: a failed run leaves no .bai.
+int do_index(const Opt& o) {
+  if (o.hostdecode) { fprintf(stderr, "index: -hostdecode is not available (the index is built from the GPU decoder's records)\n"); return 2; }
+  std::string err; long long coff = 0, skip = 0;
+  BamHeader h;
+  if (!read_bam_header(o.bamfile, &h, &coff, &skip, &err)) { fprintf(stderr, "%s\n", err.c_str()); return 1; }
+  const std::string out = o.out_set ? o.outfile : o.bamfile + ".bai";
+  const std::string tmp = out + ".tmp." + std::to_string((long long)getpid());
+  rsigpu_ctx* dec = nullptr;
+  if (create_decoder(o, 0, &dec)) { fprintf(stderr, "cannot create the decoder context\n"); return 2; }
+  int rc = 1;
+  const double t0 = now_s();
+  DecodeTiming tm;
+  if (rsigpu_bam_begin(dec, (int32_t)h.name.size()) || rsigpu_bam_index_begin(dec, (int64_t)coff)) fprintf(stderr, "%s\n", rsigpu_last_error(dec));
+  else if (stream_bam(o.bamfile, coff, skip, 0, dec, (size_t)256 << 20, [](int, const rsigpu_bam_run&) { return 0; }, &tm) == 0) {
+    int64_t nb = 0;
+    std::vector<uint8_t> ix;
+    if (rsigpu_bam_index_get(dec, nullptr, 0, &nb) == 0) { ix.resize((size_t)nb); if (rsigpu_bam_index_get(dec, ix.data(), nb, &nb)) ix.clear(); }
+    if (ix.empty()) fprintf(stderr, "%s\n", rsigpu_last_error(dec));
+    else {
+      FILE* f = fopen(tmp.c_str(), "wb");
+      const bool ok = f && fwrite(ix.data(), 1, ix.size(), f) == ix.size();
+      if (f && fclose(f) != 0) rc = 1;
+      if (ok && rename(tmp.c_str(), out.c_str()) == 0) rc = 0;
+      else fprintf(stderr, "cannot write %s\n", out.c_str());
+    }
+  }
+  if (rc) unlink(tmp.c_str());
+  rsigpu_destroy(dec);
+  if (getenv("RSICNV_TIMING")) fprintf(stderr, "#timing: index %.3f s (read %.3f, bam_feed %.3f)\n", now_s() - t0, tm.read, tm.feed);
+  return rc;
+}
+
 int do_decode(const Opt& o) {
   BamReader br(o.threads); std::string err;
   {   // what the GPU decoder is given: where the alignment records start
@@ -780,6 +818,7 @@ int main(int argc, char** argv) {
   const double t_main = now_s();
   const int ndev = rsigpu_num_devices();
   if (ndev <= 0) { fprintf(stderr, "no CUDA device: this implementation has no CPU path\n"); return 2; }
+  if (o.function == "index") return do_index(o);
   if (o.split > 1) {
     if (o.split > ndev) { fprintf(stderr, "-split %d: only %d GPUs\n", o.split, ndev); return 2; }
     if (o.hostdecode || o.saverd) { fprintf(stderr, "-split works with the GPU decoder and without -s\n"); return 2; }
