@@ -136,7 +136,9 @@ int rsigpu_pileup_commit(rsigpu_ctx* c);   /* only marks the staged batches comp
  *                                   more of the file).  `skip` = decoded bytes in front of the first record (first
  *                                   feed only).  Records are decoded into device arrays owned by the decoder and
  *                                   reported as runs of consecutive records with the same refID, in file order; a
- *                                   record cut by the end of the chunk is carried into the next feed.
+ *                                   record cut by the end of the chunk is carried into the next feed, and on through
+ *                                   as many feeds as it spans (a carried record may be up to 16 MiB: RSIGPU_E_RANGE,
+ *                                   naming its size, beyond that).
  *   take(c, run, dst)               appends the run's records to dst's staged reads, exactly as rsigpu_pileup_push
  *                                   of the same records would (dst: set_reference + pileup_begin done; dst may be c
  *                                   itself or a context on another GPU).  Runs are valid until the next feed.

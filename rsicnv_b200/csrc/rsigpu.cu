@@ -784,11 +784,18 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
       c->b_runs.push_back(R);
     }
   }
-  // the record cut by the end of this chunk is kept for the next feed (it goes in front of that chunk's first block)
+  // the record cut by the end of this chunk is kept for the next feed (it goes in front of that chunk's first block); a record
+  // that began in the carry and still does not end here (tail_start < BAM_HEAD) is carried again, however many feeds it spans
   const i64 tail_len = (i64)(BAM_HEAD + utotal) - tail_start;
   if (multi && tail_len > 0) { c->fail("bam_feed_parts: the last part ends inside a record"); return RSIGPU_E_ARG; }
   if (tail_len > 0) {
-    if (tail_start < (i64)BAM_HEAD || tail_len > (i64)BAM_HEAD) { c->fail("bam_feed: an alignment record longer than the decoder's carry buffer (16 MiB)"); return RSIGPU_E_RANGE; }
+    if (tail_len > (i64)BAM_HEAD) {
+      u32 bs = 0;                        // the record's block_size: its first 4 bytes are decoded
+      CK(cudaMemcpyAsync(&bs, c->b_U.p + tail_start, 4, cudaMemcpyDeviceToHost, c->stream));
+      CK(cudaStreamSynchronize(c->stream));
+      c->fail("bam_feed: an alignment record of " + std::to_string((u64)bs + 4) + " bytes, longer than the decoder's carry buffer (16 MiB)");
+      return RSIGPU_E_RANGE;
+    }
     CK(c->b_carry.ensure((size_t)BAM_HEAD));
     CK(cudaMemcpyAsync(c->b_carry.p, c->b_U.p + tail_start, (size_t)tail_len, cudaMemcpyDeviceToDevice, c->stream));
     CK(cudaStreamSynchronize(c->stream));
@@ -816,7 +823,7 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
       for (int w = L.w0; w <= L.w1; ++w) lin[(size_t)w] = L.voff;
     }
     if (n) { c->ix_has_prev = true; c->ix_prev_tid = (int)(u32)xc[BIX_C_LAST_TID]; c->ix_prev_pos = (int)(u32)xc[BIX_C_LAST_POS]; c->ix_prev_bin = (u32)xc[BIX_C_LAST_BIN]; c->ix_prev_key = xc[BIX_C_MAXKEY]; }
-    if (tail_len > 0) c->ix_carry_voff = voff_at(tail_start);
+    if (tail_len > 0 && tail_start >= (i64)BAM_HEAD) c->ix_carry_voff = voff_at(tail_start);   // else: the carried record began in an earlier feed
     // where the stream stops if this is the last feed: an empty block at the end (the EOF marker) is that place, else the byte after the chunk
     const i64 u_end = (i64)(BAM_HEAD + utotal);
     c->ix_end_voff = bound[(size_t)nblk - 1] == u_end ? voff_at(u_end) : (u64)(c->ix_off + (int64_t)off) << 16;

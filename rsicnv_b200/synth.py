@@ -326,6 +326,70 @@ def make_reads(L: int, seed: int, fasta: np.ndarray | None = None, coverage: flo
     return reads, events
 
 
+def make_long_reads(L: int, n: int, seed: int, tid: int = 0, max_ops: int = 200, max_len: int = 50_000, max_skip: int = 500_000,
+                    max_other: int = 300, min_len: int = 0):
+    """Long, spliced and many-op reads, unlike make_reads' 2x100 bp pairs: 1..max_ops CIGAR ops of every type 0-8 in any order
+    (so I/S/N/H/P can precede the first M/D/=/X op and S can sit between M ops), lengths log-uniform -- M/=/X in
+    [min_len, max_len], N up to max_skip, the rest up to max_other; zero-length ops included when min_len is 0.  Qualities
+    0-255, mapq 0-60, FR / proper / duplicate / secondary flags at random.  Positions uniform in [0, L), plus reads at 0 and at
+    L - 1; many reads reach past L.  Each read has exactly as many qualities as its CIGAR consumes query bases (M/I/S/=/X).
+    Returns the position-sorted SoA dict that pileup_push, write_bam and the oracle bindings take."""
+    rng = np.random.default_rng(seed + 7000)
+
+    def logu(lo, hi, size):        # integers in [lo, hi], log-uniform: mostly short, a few near hi
+        return np.minimum(lo + np.floor(np.expm1(rng.random(size) * np.log1p(hi - lo + 1))).astype(np.int64), hi)
+    nops = rng.integers(1, max_ops + 1, n)
+    op = rng.integers(0, 9, int(nops.sum()))
+    ln = np.where(np.isin(op, (0, 7, 8)), logu(min_len, max_len, len(op)),
+                  np.where(op == 3, logu(0, max_skip, len(op)), logu(0, max_other, len(op))))
+    cigar_off = np.concatenate(([0], np.cumsum(nops))).astype(np.uint32)
+    cigar = ((ln.astype(np.uint32) << 4) | op.astype(np.uint32)).astype(np.uint32)
+    qcons = np.where(np.isin(op, (0, 1, 4, 7, 8)), ln, 0)
+    qlen = np.add.reduceat(qcons, cigar_off[:-1].astype(np.int64))
+    qual_off = np.concatenate(([0], np.cumsum(qlen))).astype(np.uint64)
+    pos = rng.integers(0, L, n).astype(np.int64)
+    pos[:min(n, 2)] = 0
+    if n > 2:
+        pos[2] = L - 1
+    order = np.argsort(pos, kind="stable")
+    flag = (rng.choice(np.array([F_PAIRED | F_MREV | F_R1, F_PAIRED | F_REV | F_R2], np.uint16), n) |
+            np.where(rng.random(n) < 0.5, F_PROPER, 0)).astype(np.uint16)
+    u = rng.random(n)
+    flag[u < 0.05] |= F_DUP
+    flag[(u >= 0.05) & (u < 0.08)] |= F_SECONDARY
+    isize = rng.integers(-2000, 2000, n).astype(np.int32)
+    R = dict(pos=pos.astype(np.int32), mpos=(pos + rng.integers(-5000, 5000, n)).clip(0, L - 1).astype(np.int32), isize=isize,
+             mtid=np.full(n, tid, np.int32), flag=flag, mapq=rng.integers(0, 61, n).astype(np.uint8), cigar_off=cigar_off,
+             cigar=cigar, qual_off=qual_off, qual=rng.integers(0, 256, int(qual_off[-1])).astype(np.uint8))
+    return take_reads(R, order)
+
+
+def take_reads(R: dict, idx) -> dict:
+    """the reads R[idx] (any order) as a new SoA dict with its own CIGAR / quality offsets"""
+    idx = np.asarray(idx, np.int64)
+    co = R["cigar_off"].astype(np.int64); qo = R["qual_off"].astype(np.int64)
+    nc = co[idx + 1] - co[idx]; nq = qo[idx + 1] - qo[idx]
+    out = {k: np.asarray(R[k])[idx] for k in ("pos", "mpos", "isize", "mtid", "flag", "mapq")}
+    out["cigar_off"] = np.concatenate(([0], np.cumsum(nc))).astype(np.uint32)
+    out["qual_off"] = np.concatenate(([0], np.cumsum(nq))).astype(np.uint64)
+    ci = np.repeat(co[idx], nc) + (np.arange(int(nc.sum())) - np.repeat(np.cumsum(nc) - nc, nc))
+    qi = np.repeat(qo[idx], nq) + (np.arange(int(nq.sum())) - np.repeat(np.cumsum(nq) - nq, nq))
+    out["cigar"] = R["cigar"][ci]; out["qual"] = R["qual"][qi]
+    return out
+
+
+def merge_reads(*sets: dict) -> dict:
+    """several read SoA dicts of one contig as one, sorted by position (stable: equal positions keep the order of `sets`)"""
+    keys = ("pos", "mpos", "isize", "mtid", "flag", "mapq", "cigar", "qual")
+    cat = {k: np.concatenate([s[k] for s in sets]) for k in keys}
+    nco = [0]; nqo = [0]
+    for s in sets:
+        nco.append(nco[-1] + int(s["cigar_off"][-1])); nqo.append(nqo[-1] + int(s["qual_off"][-1]))
+    cat["cigar_off"] = np.concatenate([s["cigar_off"][:-1].astype(np.int64) + b for s, b in zip(sets, nco)] + [[nco[-1]]]).astype(np.uint32)
+    cat["qual_off"] = np.concatenate([s["qual_off"][:-1].astype(np.int64) + b for s, b in zip(sets, nqo)] + [[nqo[-1]]]).astype(np.uint64)
+    return take_reads(cat, np.argsort(cat["pos"], kind="stable"))
+
+
 def _fill_var(buf, starts, lens, values):
     """buf[starts[r] + k] = values[...] for k < lens[r], all records at once"""
     lens = np.asarray(lens, np.int64)
