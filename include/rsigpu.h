@@ -125,6 +125,21 @@ int rsigpu_pileup_begin(rsigpu_ctx* c, int32_t target_len);
 int rsigpu_pileup_push(rsigpu_ctx* c, const rsigpu_read_batch* b);
 int rsigpu_pileup_end(rsigpu_ctx* c);      /* runs the pileup kernels now: the raw depth becomes readable (-s) */
 int rsigpu_pileup_commit(rsigpu_ctx* c);   /* only marks the staged batches complete; rsigpu_run runs the pileup as its first stage */
+/* Reads that are not in position order (a BAM that is not coordinate-sorted, records gathered from several feeds):
+ *   pileup_sort(c)               sorts the staged reads by pos on the GPU, stable (reads at one position keep their staging
+ *                                order), fixed fields, CIGAR ops and qualities.  Reads already in position order cost only the
+ *                                sortedness check the pileup runs anyway.  Afterwards rsigpu_run, rsigpu_pileup_end and
+ *                                rsigpu_stat_calls take them as they take sorted input.  The sort needs a second copy of the
+ *                                staged reads in HBM, plus 16 B per read of sort keys and indices, while it runs, and releases
+ *                                both before it returns (RSIGPU_E_CUDA when there is no room: the reads are unchanged).
+ *   reads_take(src, r0, r1, dst) appends src's staged reads [r0, r1) to dst's staged reads, exactly as rsigpu_pileup_push of the
+ *                                same reads would (dst: set_reference + pileup_begin or reads_begin done; dst != src; dst may
+ *                                be on another GPU).
+ *   reads_field(c, field, ...)   one field of ALL staged reads copied to the host, numbered as in rsigpu_bam_run_field;
+ *                                out == NULL or cap_bytes < *nbytes: only *nbytes. */
+int rsigpu_pileup_sort(rsigpu_ctx* c);
+int rsigpu_reads_take(rsigpu_ctx* src, int64_t r0, int64_t r1, rsigpu_ctx* dst);
+int rsigpu_reads_field(rsigpu_ctx* c, int32_t field, void* out, int64_t cap_bytes, int64_t* nbytes);
 
 /* BAM input straight from the file's bytes: BGZF inflate (samtools-0.1.18/bgzf.c:277-313 inflate_block,
  * 258-275 check_header) and bam_read1 (bam.c:179-210, core layout bam.h:131-155) on the GPU.  The caller
@@ -261,6 +276,18 @@ int rsigpu_set_inflate_mode(rsigpu_ctx* c, int mode);
  *   "bam_feed_parts: CRC32 mismatch in BGZF block <k> of part <j> (compressed offset <X> of that part)"
  * A block whose deflate stream is corrupt is still reported as such; a CRC mismatch is reported before a corrupt record. */
 int rsigpu_set_bgzf_crc(rsigpu_ctx* c, int on);
+/* on != 0: every rsigpu_bam_feed sorts its complete records by refID on the GPU, stable in file order, before it reports the
+ * runs: a feed then reports at most one run per refID present, in increasing refID order with the unplaced records (refID -1)
+ * last, and each run holds its records in file order.  A record carried across feeds belongs to the feed it completes in.
+ * This is what a file that is not coordinate-sorted needs (without it, such a file fails with "more than 65536 refID runs"):
+ * gather each reference's runs over all feeds (rsigpu_bam_take into one staging context, rsigpu_reads_take), then
+ * rsigpu_pileup_sort.  Default 0: nothing of this runs.  Refused with RSIGPU_E_ARG, naming the conflict:
+ *   rsigpu_bam_index_begin while on, and set_bam_by_ref(c, 1) while an index is built (the index needs file order);
+ *   rsigpu_bam_feed_parts while on (each part already starts its own run);
+ *   rsigpu_bam_take_range on a run grouped by refID (its positions are not sorted);
+ *   more than 65535 references (rsigpu_bam_begin, or set_bam_by_ref after it): one run per reference and refID -1 must fit
+ *   the 65536 runs of a feed. */
+int rsigpu_set_bam_by_ref(rsigpu_ctx* c, int on);
 /* tuning hook: threads of the bin-level candidate kernel (multiple of 32, 32..1024) */
 int rsigpu_set_cand_threads(rsigpu_ctx* c, int threads);
 /* test hook: selected device-resident scalars of the last stage, as doubles; returns how many exist */

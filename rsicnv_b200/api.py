@@ -72,7 +72,8 @@ EXPORTS = ("rsigpu_default_params", "rsigpu_create", "rsigpu_destroy", "rsigpu_l
            "rsigpu_sd_filters", "rsigpu_cnv_stat", "rsigpu_get_calls", "rsigpu_run", "rsigpu_get_chr_stats", "rsigpu_get_array",
            "rsigpu_format_row", "rsigpu_launch_count", "rsigpu_last_stage_ms", "rsigpu_set_profile", "rsigpu_get_profile",
            "rsigpu_get_log", "rsigpu_reads_begin", "rsigpu_stat_calls", "rsigpu_bam_take_range", "rsigpu_split_range", "rsigpu_split_run", "rsigpu_split_p2p_bytes", "rsigpu_set_level0_mode", "rsigpu_set_feed_limit", "rsigpu_set_inflate_mode", "rsigpu_set_bgzf_crc", "rsigpu_set_cand_threads", "rsigpu_debug_state", "rsigpu_pileup_commit", "rsigpu_bam_begin", "rsigpu_bam_feed", "rsigpu_bam_feed_parts", "rsigpu_bam_take",
-           "rsigpu_bam_end", "rsigpu_bam_run_field", "rsigpu_bam_index_begin", "rsigpu_bam_index_get", "rsigpu_pinned_alloc", "rsigpu_pinned_free")
+           "rsigpu_bam_end", "rsigpu_bam_run_field", "rsigpu_bam_index_begin", "rsigpu_bam_index_get", "rsigpu_pinned_alloc", "rsigpu_pinned_free",
+           "rsigpu_set_bam_by_ref", "rsigpu_pileup_sort", "rsigpu_reads_take", "rsigpu_reads_field")
 
 _libs: dict[str, C.CDLL] = {}
 
@@ -315,6 +316,35 @@ class Context:
                 self._ck(self.lib.rsigpu_bam_run_field(self.h, C.c_int32(run), C.c_int32(f), _ptr(a), C.c_int64(nb.value), C.byref(nb)))
             out[name] = a
         return out
+
+    def reads(self) -> dict:
+        """every staged read as the read dict pileup_push takes (rsigpu_reads_field)"""
+        out = {}
+        for f, (name, dt) in enumerate(self._BAM_FIELDS):
+            nb = C.c_int64(0)
+            self._ck(self.lib.rsigpu_reads_field(self.h, C.c_int32(f), None, C.c_int64(0), C.byref(nb)))
+            a = np.empty(nb.value // np.dtype(dt).itemsize, dt)
+            if nb.value:
+                self._ck(self.lib.rsigpu_reads_field(self.h, C.c_int32(f), _ptr(a), C.c_int64(nb.value), C.byref(nb)))
+            out[name] = a
+        return out
+
+    def reads_take(self, r0: int, r1: int, dst: "Context"):
+        """append this context's staged reads [r0, r1) to dst's (rsigpu_reads_take)"""
+        before = (self.lib.rsigpu_last_error(self.h), self.lib.rsigpu_last_error(dst.h))
+        rc = self.lib.rsigpu_reads_take(self.h, C.c_int64(r0), C.c_int64(r1), dst.h)
+        if rc != 0:   # the message of whichever context the failure was recorded on (a stale one on the other is ignored)
+            src_e, dst_e = self.lib.rsigpu_last_error(self.h), self.lib.rsigpu_last_error(dst.h)
+            msg = src_e if src_e and src_e != before[0] else dst_e if dst_e and dst_e != before[1] else src_e or dst_e or b""
+            raise RsiGpuError(rc, msg.decode())
+
+    def pileup_sort(self):
+        """sort the staged reads by position on the GPU, stable (rsigpu_pileup_sort)"""
+        self._ck(self.lib.rsigpu_pileup_sort(self.h))
+
+    def set_bam_by_ref(self, on: bool):
+        """group each bam_feed's records by refID, -1 last, stable in file order (rsigpu_set_bam_by_ref)"""
+        self._ck(self.lib.rsigpu_set_bam_by_ref(self.h, C.c_int(1 if on else 0)))
 
     def reads_begin(self, tid: int, target_len: int):
         """`stat`: stage reads of one contig without a reference (then pileup_push / bam_take)"""

@@ -22,6 +22,7 @@
 #include "k_bam.cuh"
 #include "k_crc32.cuh"
 #include "k_bam_index.cuh"
+#include "k_sort.cuh"
 
 using namespace rsigpu;
 
@@ -69,6 +70,13 @@ struct DevVec {   // growable device array filled by appends from the host
   }
   void clear() { n = 0; }
   void release() { if (p) cudaFree(p); p = nullptr; n = cap = 0; }
+  // a fresh array of exactly cnt elements (contents undefined), replacing this one
+  cudaError_t alloc_exact(size_t cnt) {
+    release();
+    cudaError_t e = cudaMalloc((void**)&p, cnt * sizeof(T) + 64);
+    if (e == cudaSuccess) { n = cnt; cap = cnt; }
+    return e;
+  }
 };
 
 const int LIST_CAP = 65536;          // runs / segments / calls per contig
@@ -153,12 +161,16 @@ struct rsigpu_ctx {
   DevBuf<u8> b_comp, b_U, b_carry, b_mapq, b_qual; DevBuf<BgzfBlock> b_blk; DevBuf<u16> b_flag, b_tabs; DevBuf<u32> b_cigoff, b_cig; DevBuf<u64> b_qoff;
   DevBuf<int> b_cnt, b_ncig, b_rbase, b_cbase, b_cnt32, b_runstart, b_tid, b_pos, b_mpos, b_isize, b_mtid;
   DevBuf<i64> b_bound, b_first, b_endp, b_tailp, b_in, b_info, b_rec, b_nq, b_qbase, b_runinfo;
-  struct BamRun { int tid, part; i64 r0, r1, c0, c1, q0, q1; };
+  struct BamRun { int tid, part; i64 r0, r1, c0, c1, q0, q1; bool by_ref; };
   std::vector<BamRun> b_runs;
   int b_nref = 0, b_tail_len = 0, b_rewalked = 0; bool b_active = false, b_first_feed = true;
   size_t b_umax = (size_t)5 << 30;   // decoded bytes one feed may produce (test hook: rsigpu_set_feed_limit)
   int inflate_mode = 0;              // 0 = by chunk size, 1 = one lane per BGZF block, 2 = one warp per BGZF block (rsigpu_set_inflate_mode)
   bool bgzf_crc = false;             // check every block's CRC32 after inflate (rsigpu_set_bgzf_crc)
+  bool bam_by_ref = false;           // group each feed's records by refID before the runs are found (rsigpu_set_bam_by_ref)
+  DevBuf<i64> b2_rec; DevBuf<int> b2_tid, b2_pos, b2_mpos, b2_isize, b2_mtid; DevBuf<u16> b2_flag; DevBuf<u8> b2_mapq; DevBuf<u32> b2_cigoff; DevBuf<u64> b2_qoff;
+  // radix sort scratch (k_sort.cuh): keys and indices ping-pong, per-tile digit counts, digit totals, offset-scan tile sums
+  DevBuf<u32> t_key, t_key2, t_idx, t_idx2, t_hist, t_dtot; DevBuf<u64> t_ts;
   // BAI index built from the decoded records (k_bam_index.cuh, rsigpu_bam_index_begin / _get)
   struct IxChunk { u32 bin; u64 u, v; };
   struct IxRef { std::vector<IxChunk> ch; u64 n_map = 0, n_unmap = 0; std::vector<u64> lin; };
@@ -413,6 +425,8 @@ void rsigpu_destroy(rsigpu_ctx* c) {
   c->b_bound.release(); c->b_first.release(); c->b_endp.release(); c->b_tailp.release(); c->b_cnt.release(); c->b_ncig.release(); c->b_in.release(); c->b_rbase.release(); c->b_cbase.release();
   c->b_info.release(); c->b_runstart.release(); c->b_rec.release(); c->b_tid.release(); c->b_pos.release(); c->b_mpos.release(); c->b_isize.release(); c->b_mtid.release();
   c->b_nq.release(); c->b_qbase.release(); c->b_runinfo.release();
+  c->b2_rec.release(); c->b2_tid.release(); c->b2_pos.release(); c->b2_mpos.release(); c->b2_isize.release(); c->b2_mtid.release(); c->b2_flag.release(); c->b2_mapq.release(); c->b2_cigoff.release(); c->b2_qoff.release();
+  c->t_key.release(); c->t_key2.release(); c->t_idx.release(); c->t_idx2.release(); c->t_hist.release(); c->t_dtot.release(); c->t_ts.release();
   c->x_beg.release(); c->x_key.release(); c->x_cnt.release(); c->x_tkey.release(); c->x_meta.release(); c->x_tstart.release(); c->x_tunmap.release(); c->x_chunk.release(); c->x_lin.release();
   if (c->d_st) cudaFree(c->d_st);
   if (c->h_st) cudaFreeHost(c->h_st);
@@ -536,9 +550,44 @@ int rsigpu_pileup_push(rsigpu_ctx* c, const rsigpu_read_batch* b) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// stable sort of read records (k_sort.cuh)
+// LSD radix sort of the n keys in c->t_key over their low `bits` bits, stable in index order; *perm: the sorted order
+static int sort_keys(rsigpu_ctx* c, u32 n, int bits, const u32** perm) {
+  const u32 ntile = (n + SRT_TILE - 1) / SRT_TILE;
+  CK(c->t_key2.ensure(n)); CK(c->t_idx.ensure(n)); CK(c->t_idx2.ensure(n)); CK(c->t_hist.ensure((size_t)SRT_RADIX * ntile)); CK(c->t_dtot.ensure(SRT_RADIX));
+  u32 *ki = c->t_key.p, *ko = c->t_key2.p, *ii = nullptr, *io = c->t_idx.p;
+  const int passes = std::max(1, (bits + SRT_BITS - 1) / SRT_BITS);
+  for (int p = 0; p < passes; ++p) {
+    KL(k_sort_hist, ntile, SRT_NT, 0, ki, n, p * SRT_BITS, c->t_hist.p, ntile);
+    KL(k_sort_scan_rows, SRT_RADIX, SRT_NT, 0, c->t_hist.p, ntile, c->t_dtot.p);
+    KL(k_sort_scatter, ntile, SRT_NT, 0, ki, ii, n, p * SRT_BITS, c->t_hist.p, c->t_dtot.p, ntile, ko, io);
+    std::swap(ki, ko);
+    ii = io; io = io == c->t_idx.p ? c->t_idx2.p : c->t_idx.p;
+  }
+  *perm = ii;
+  return RSIGPU_OK;
+}
+// lc[0..n) / lq[0..n) hold lengths: exclusive prefix sums in place, the totals to lc[n] / lq[n] (n > 0)
+static int lengths_to_offsets(rsigpu_ctx* c, u32* lc, u64* lq, u32 n) {
+  const u32 ntile = (n + OFS_TILE - 1) / OFS_TILE;
+  CK(c->t_ts.ensure(2 * (size_t)ntile));
+  KL(k_off_tile_sums, ntile, OFS_NT, 0, lc, lq, n, c->t_ts.p, ntile);
+  KL(k_off_tile_scan, 1, 1024, 0, c->t_ts.p, ntile, lc, lq, n);
+  KL(k_off_apply, ntile, OFS_NT, 0, lc, lq, n, c->t_ts.p, ntile);
+  return RSIGPU_OK;
+}
+static int bit_width(u32 v) { int b = 0; while (v) { ++b; v >>= 1; } return b; }
+
+// ---------------------------------------------------------------------------------------------
 // BAM bytes -> staged reads on the GPU (k_bam.cuh)
+const int BY_REF_MAX_REFS = LIST_CAP - 1;   // with refID -1, one run per reference must fit a feed's run list
+
 int rsigpu_bam_begin(rsigpu_ctx* c, int32_t n_ref) {
   if (!c || n_ref < 1) return RSIGPU_E_ARG;
+  if (c->bam_by_ref && n_ref > BY_REF_MAX_REFS) {
+    c->fail("bam_begin: " + std::to_string(n_ref) + " references, more than the 65535 that grouping records by refID (rsigpu_set_bam_by_ref) supports");
+    return RSIGPU_E_ARG;
+  }
   c->b_nref = n_ref; c->b_tail_len = 0; c->b_active = true; c->b_first_feed = true; c->b_runs.clear(); c->b_rewalked = 0;
   c->ix_on = false; c->ix_failed = false; c->ix_ready = false; c->ix_out.clear(); c->ix_ref.clear();
   return RSIGPU_OK;
@@ -546,6 +595,7 @@ int rsigpu_bam_begin(rsigpu_ctx* c, int32_t n_ref) {
 
 int rsigpu_bam_index_begin(rsigpu_ctx* c, int64_t file_offset) {
   if (!c) return RSIGPU_E_ARG;
+  if (c->bam_by_ref) { c->fail("bam_index_begin: not available while records are grouped by refID (rsigpu_set_bam_by_ref): the index needs them in file order"); return RSIGPU_E_ARG; }
   if (!c->b_active || !c->b_first_feed || file_offset < 0) { c->fail("bam_index_begin: call it after rsigpu_bam_begin and before the first feed, with the file offset of the first byte fed"); return RSIGPU_E_ARG; }
   c->ix_on = true; c->ix_failed = false; c->ix_ready = false; c->ix_has_prev = false; c->ix_off = file_offset;
   c->ix_carry_voff = 0; c->ix_end_voff = 0; c->ix_prev_key = 0; c->ix_no_coor = 0; c->ix_pend_on = false; c->ix_pend_tid = -1;
@@ -712,6 +762,25 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
     BamSoA S; S.rec = c->b_rec.p; S.tid = c->b_tid.p; S.pos = c->b_pos.p; S.mpos = c->b_mpos.p; S.isize = c->b_isize.p; S.mtid = c->b_mtid.p; S.flag = c->b_flag.p;
     S.mapq = c->b_mapq.p; S.cigar_off = c->b_cigoff.p; S.cigar = c->b_cig.p; S.qual_off = c->b_qoff.p; S.qual = c->b_qual.p;
     KL(k_bam_fields, (nblk + 127) / 128, 128, 0, C, H, c->b_rbase.p, c->b_cbase.p, c->b_qbase.p, info, S);
+    if (c->bam_by_ref) {
+      // the records grouped by refID, stable in file order (k_sort.cuh): the fixed fields and the offsets move, and
+      // k_bam_payload then copies every record's CIGAR and qualities from the inflated bytes straight to its sorted place
+      CK(c->t_key.ensure(n)); CK(c->b2_rec.ensure(n)); CK(c->b2_tid.ensure(n)); CK(c->b2_pos.ensure(n)); CK(c->b2_mpos.ensure(n)); CK(c->b2_isize.ensure(n));
+      CK(c->b2_mtid.ensure(n)); CK(c->b2_flag.ensure(n)); CK(c->b2_mapq.ensure(n)); CK(c->b2_cigoff.ensure(n + 1)); CK(c->b2_qoff.ensure(n + 1));
+      const int g = grid_for((int)n, 1024, c->n_sm * 8);
+      KL(k_sort_key_tid, g, 256, 0, c->b_tid.p, (u32)n, (u32)c->b_nref, c->t_key.p);
+      const u32* perm = nullptr;
+      int rc = sort_keys(c, (u32)n, bit_width((u32)c->b_nref), &perm);
+      if (rc) return rc;
+      SortFields fi{c->b_rec.p, c->b_tid.p, c->b_pos.p, c->b_mpos.p, c->b_isize.p, c->b_mtid.p, c->b_flag.p, c->b_mapq.p, c->b_cigoff.p, c->b_qoff.p};
+      SortFields fo{c->b2_rec.p, c->b2_tid.p, c->b2_pos.p, c->b2_mpos.p, c->b2_isize.p, c->b2_mtid.p, c->b2_flag.p, c->b2_mapq.p, c->b2_cigoff.p, c->b2_qoff.p};
+      KL(k_sort_gather, g, 256, 0, perm, (u32)n, fi, fo);
+      if ((rc = lengths_to_offsets(c, c->b2_cigoff.p, c->b2_qoff.p, (u32)n))) return rc;
+      std::swap(c->b_rec, c->b2_rec); std::swap(c->b_tid, c->b2_tid); std::swap(c->b_pos, c->b2_pos); std::swap(c->b_mpos, c->b2_mpos); std::swap(c->b_isize, c->b2_isize);
+      std::swap(c->b_mtid, c->b2_mtid); std::swap(c->b_flag, c->b2_flag); std::swap(c->b_mapq, c->b2_mapq); std::swap(c->b_cigoff, c->b2_cigoff); std::swap(c->b_qoff, c->b2_qoff);
+      S.rec = c->b_rec.p; S.tid = c->b_tid.p; S.pos = c->b_pos.p; S.mpos = c->b_mpos.p; S.isize = c->b_isize.p; S.mtid = c->b_mtid.p; S.flag = c->b_flag.p;
+      S.mapq = c->b_mapq.p; S.cigar_off = c->b_cigoff.p; S.qual_off = c->b_qoff.p;
+    }
     KL(k_bam_payload, c->n_sm * 8, 256, 0, c->b_U.p, info, S);
     KL(k_bam_runs, grid_for((int)std::min<size_t>(n, 1u << 30), 1024, c->n_sm * 8), 256, 0, c->b_tid.p, info, c->b_runstart.p, (int)LIST_CAP, err);
     if (c->ix_on) {          // the BAI index's share of this feed (k_bam_index.cuh); its counts travel with the error copy below
@@ -778,7 +847,7 @@ static int bam_feed_impl(rsigpu_ctx* c, int nparts, const uint8_t* const* ptrs, 
     CK(cudaStreamSynchronize(c->stream));
     for (int i = 0; i < nr; ++i) {
       rsigpu_ctx::BamRun R; R.tid = (int)ri[3 * (size_t)i]; R.r0 = rs[(size_t)i]; R.c0 = ri[3 * (size_t)i + 1]; R.q0 = ri[3 * (size_t)i + 2];
-      R.part = 0;
+      R.part = 0; R.by_ref = c->bam_by_ref;
       if (multi) { while (R.part + 1 < nparts && part_rec[(size_t)R.part + 1] <= rs[(size_t)i] && part_blk[(size_t)R.part + 1] < nblk) ++R.part; }
       R.r1 = i + 1 < nr ? rs[(size_t)i + 1] : (i64)n; R.c1 = i + 1 < nr ? ri[3 * (size_t)i + 4] : (i64)ncg; R.q1 = i + 1 < nr ? ri[3 * (size_t)i + 5] : nq64;
       c->b_runs.push_back(R);
@@ -845,6 +914,7 @@ int rsigpu_bam_feed(rsigpu_ctx* c, const uint8_t* bgzf, int64_t nbytes, int64_t 
 }
 int rsigpu_bam_feed_parts(rsigpu_ctx* c, int32_t n_parts, const uint8_t* const* parts, const int64_t* nbytes, rsigpu_bam_run* runs, int32_t cap, int32_t* n_runs) {
   if (n_parts < 1) return RSIGPU_E_ARG;
+  if (c && c->bam_by_ref) { c->fail("bam_feed_parts: not available while records are grouped by refID (rsigpu_set_bam_by_ref): each part already starts its own run"); return RSIGPU_E_ARG; }
   if (c && c->ix_on) { c->ix_failed = true; c->fail("bam_feed_parts: not available while a BAM index is built (rsigpu_bam_index_begin): its parts are not one contiguous file"); return RSIGPU_E_ARG; }
   if (n_parts == 1) { int64_t consumed = 0; const int rc = bam_feed_impl(c, 1, parts, nbytes, 0, &consumed, runs, cap, n_runs); if (rc == RSIGPU_OK && consumed != nbytes[0]) { c->fail("bam_feed_parts: a part is not a whole number of BGZF blocks"); return RSIGPU_E_RANGE; } return rc; }
   return bam_feed_impl(c, n_parts, parts, nbytes, 0, nullptr, runs, cap, n_runs);
@@ -867,6 +937,7 @@ int rsigpu_bam_take_range(rsigpu_ctx* c, int32_t run, rsigpu_ctx* dst, int32_t p
   if (!c || !dst || run < 0 || run >= (int)c->b_runs.size()) return RSIGPU_E_ARG;
   if (!dst->have_ref) { dst->fail("bam_take: call set_reference and pileup_begin on the destination first"); return RSIGPU_E_ARG; }
   const rsigpu_ctx::BamRun& R = c->b_runs[(size_t)run];
+  if (R.by_ref) { c->fail("bam_take_range: run " + std::to_string(run) + " was grouped by refID (rsigpu_set_bam_by_ref): its positions are not sorted"); return RSIGPU_E_ARG; }
   const long long n = R.r1 - R.r0;
   if (n == 0 || pos_hi <= pos_lo) return RSIGPU_OK;
   cudaSetDevice(c->device);
@@ -1002,6 +1073,119 @@ int rsigpu_pileup_commit(rsigpu_ctx* c) {
   if (!c) return RSIGPU_E_ARG;
   if (!c->have_ref) { c->fail("pileup_commit: call set_reference / pileup_begin first"); return RSIGPU_E_ARG; }
   c->have_reads = true; c->have_depth = false; c->loaded = false; c->detected = false; c->filtered = false;
+  return RSIGPU_OK;
+}
+
+int rsigpu_pileup_sort(rsigpu_ctx* c) {
+  if (!c) return RSIGPU_E_ARG;
+  if (!c->have_ref) { c->fail("pileup_sort: call set_reference and pileup_begin (or reads_begin) first"); return RSIGPU_E_ARG; }
+  const size_t n = c->r_pos.n;
+  if (n < 2) return RSIGPU_OK;
+  if (n > 0x7fffffffull) { c->fail("pileup_sort: more than 2^31 - 1 staged reads"); return RSIGPU_E_RANGE; }
+  cudaSetDevice(c->device);
+  // the check the pileup runs anyway (k_read_ends' sorted_bad): reads already in position order cost nothing more
+  CK(c->r_calend.ensure(n + 8)); CK(c->r_ncig.ensure(n + 8));
+  int* mx = c->d_misc.p + 5;   // max_extent, sorted_bad
+  if (c->isize_pending) { CK(cudaStreamWaitEvent(c->stream, c->ev_isize, 0)); c->isize_pending = false; }
+  CK(cudaMemsetAsync(mx, 0, 8, c->stream));
+  KL(k_read_ends, grid_for((int)std::min<size_t>(n, 1u << 30), 256, c->n_sm * 16), 256, 0, read_view(c), mx, mx + 1);
+  int bad = 0;
+  CK(cudaMemcpyAsync(&bad, mx + 1, 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  if (!bad) return RSIGPU_OK;
+  // keys pos + 1; the passes cover the bits of the largest key
+  CK(c->t_key.ensure(n)); CK(c->t_dtot.ensure(SRT_RADIX + 1));
+  u32* kmax = c->t_dtot.p + SRT_RADIX;
+  CK(cudaMemsetAsync(kmax, 0, 4, c->stream));
+  const int g = grid_for((int)n, 1024, c->n_sm * 8);
+  KL(k_sort_key_pos, g, 256, 0, c->r_pos.p, (u32)n, c->t_key.p, kmax);
+  u32 hk = 0;
+  CK(cudaMemcpyAsync(&hk, kmax, 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  const u32* perm = nullptr;
+  int rc = sort_keys(c, (u32)n, bit_width(hk), &perm);
+  if (rc) return rc;
+  // gather into fresh arrays, which then replace the staged ones
+  DevVec<int> pos, mpos, isize, mtid; DevVec<u16> flag; DevVec<u8> mapq, qual; DevVec<u32> coff, cig; DevVec<u64> qoff;
+  auto drop = [&]() { pos.release(); mpos.release(); isize.release(); mtid.release(); flag.release(); mapq.release(); qual.release(); coff.release(); cig.release(); qoff.release(); };
+  cudaError_t e = pos.alloc_exact(n);
+  if (e == cudaSuccess) e = mpos.alloc_exact(n);
+  if (e == cudaSuccess) e = isize.alloc_exact(n);
+  if (e == cudaSuccess) e = mtid.alloc_exact(n);
+  if (e == cudaSuccess) e = flag.alloc_exact(n);
+  if (e == cudaSuccess) e = mapq.alloc_exact(n);
+  if (e == cudaSuccess) e = coff.alloc_exact(n + 1);
+  if (e == cudaSuccess) e = qoff.alloc_exact(n + 1);
+  if (e == cudaSuccess) e = cig.alloc_exact(c->r_cigar.n);
+  if (e == cudaSuccess) e = qual.alloc_exact(c->r_qual.n);
+  if (e != cudaSuccess) { drop(); c->fail(std::string("pileup_sort: no device memory for the sorted copy of the reads: ") + cudaGetErrorString(e)); return RSIGPU_E_CUDA; }
+  SortFields fi{nullptr, nullptr, c->r_pos.p, c->r_mpos.p, c->r_isize.p, c->r_mtid.p, c->r_flag.p, c->r_mapq.p, c->r_cigar_off.p, c->r_qual_off.p};
+  SortFields fo{nullptr, nullptr, pos.p, mpos.p, isize.p, mtid.p, flag.p, mapq.p, coff.p, qoff.p};
+  KL(k_sort_gather, g, 256, 0, perm, (u32)n, fi, fo);
+  if ((rc = lengths_to_offsets(c, coff.p, qoff.p, (u32)n))) { drop(); return rc; }
+  KL(k_sort_gather_payload, c->n_sm * 8, 256, 0, perm, (u32)n, c->r_cigar_off.p, c->r_cigar.p, c->r_qual_off.p, c->r_qual.p, coff.p, cig.p, qoff.p, qual.p);
+  e = cudaStreamSynchronize(c->stream);
+  if (e != cudaSuccess || !c->launch_err.empty()) {
+    drop();
+    c->fail("pileup_sort: " + (e != cudaSuccess ? std::string(cudaGetErrorString(e)) : "kernel launch failed: " + c->launch_err));
+    c->launch_err.clear();
+    return RSIGPU_E_CUDA;
+  }
+  std::swap(c->r_pos, pos); std::swap(c->r_mpos, mpos); std::swap(c->r_isize, isize); std::swap(c->r_mtid, mtid); std::swap(c->r_flag, flag);
+  std::swap(c->r_mapq, mapq); std::swap(c->r_cigar_off, coff); std::swap(c->r_qual_off, qoff); std::swap(c->r_cigar, cig); std::swap(c->r_qual, qual);
+  drop();   // the unsorted arrays
+  // the sort scratch (16 B per read and the digit counts) is not kept: a context holds one contig's reads at a time
+  c->t_key.release(); c->t_key2.release(); c->t_idx.release(); c->t_idx2.release(); c->t_hist.release(); c->t_ts.release();
+  c->pileup_fresh = false;
+  return RSIGPU_OK;
+}
+
+int rsigpu_reads_take(rsigpu_ctx* src, int64_t r0, int64_t r1, rsigpu_ctx* dst) {
+  if (!src || !dst) return RSIGPU_E_ARG;
+  rsigpu_ctx* c = src;
+  if (src == dst) { c->fail("reads_take: the source and the destination are the same context"); return RSIGPU_E_ARG; }
+  if (r0 < 0 || r1 < r0 || (size_t)r1 > c->r_pos.n) {
+    c->fail("reads_take: reads [" + std::to_string(r0) + ", " + std::to_string(r1) + ") outside the " + std::to_string(c->r_pos.n) + " staged reads");
+    return RSIGPU_E_ARG;
+  }
+  if (!dst->have_ref) { dst->fail("reads_take: call set_reference and pileup_begin (or reads_begin) on the destination first"); return RSIGPU_E_ARG; }
+  if (r1 == r0) return RSIGPU_OK;
+  cudaSetDevice(c->device);
+  u32 co[2]; u64 qo[2];
+  CK(cudaMemcpyAsync(&co[0], c->r_cigar_off.p + r0, 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(&co[1], c->r_cigar_off.p + r1, 4, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(&qo[0], c->r_qual_off.p + r0, 8, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(&qo[1], c->r_qual_off.p + r1, 8, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  rsigpu_read_batch b; memset(&b, 0, sizeof b);
+  b.n_reads = r1 - r0; b.tid = c->tid;
+  b.pos = c->r_pos.p + r0; b.mpos = c->r_mpos.p + r0; b.isize = c->r_isize.p + r0; b.mtid = c->r_mtid.p + r0; b.flag = c->r_flag.p + r0; b.mapq = c->r_mapq.p + r0;
+  b.cigar_off = c->r_cigar_off.p + r0; b.cigar = c->r_cigar.p + co[0]; b.qual_off = reinterpret_cast<const uint64_t*>(c->r_qual_off.p + r0); b.qual = c->r_qual.p + qo[0];
+  return push_impl(dst, &b, (size_t)(co[1] - co[0]), (size_t)(qo[1] - qo[0]), co[0], qo[0], c->device);
+}
+
+int rsigpu_reads_field(rsigpu_ctx* c, int32_t field, void* out, int64_t cap_bytes, int64_t* nbytes) {
+  if (!c || !nbytes) return RSIGPU_E_ARG;
+  cudaSetDevice(c->device);
+  const size_t n = c->r_pos.n;
+  const void* src = nullptr; size_t bytes = 0;
+  switch (field) {
+    case 0: src = c->r_pos.p; bytes = n * 4; break;
+    case 1: src = c->r_mpos.p; bytes = n * 4; break;
+    case 2: src = c->r_isize.p; bytes = n * 4; break;
+    case 3: src = c->r_mtid.p; bytes = n * 4; break;
+    case 4: src = c->r_flag.p; bytes = n * 2; break;
+    case 5: src = c->r_mapq.p; bytes = n; break;
+    case 6: src = c->r_cigar_off.p; bytes = (n + 1) * 4; break;
+    case 7: src = c->r_cigar.p; bytes = c->r_cigar.n * 4; break;
+    case 8: src = c->r_qual_off.p; bytes = (n + 1) * 8; break;
+    case 9: src = c->r_qual.p; bytes = c->r_qual.n; break;
+    default: return RSIGPU_E_ARG;
+  }
+  *nbytes = (int64_t)bytes;
+  if (!out || cap_bytes < (int64_t)bytes) return RSIGPU_OK;
+  if (n == 0 && (field == 6 || field == 8)) { memset(out, 0, bytes); return RSIGPU_OK; }   // nothing staged: the one offset is 0
+  if (bytes) { CK(cudaMemcpyAsync(out, src, bytes, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream)); }
   return RSIGPU_OK;
 }
 
@@ -1719,6 +1903,16 @@ int rsigpu_set_inflate_mode(rsigpu_ctx* c, int mode) {
 int rsigpu_set_bgzf_crc(rsigpu_ctx* c, int on) {
   if (!c) return RSIGPU_E_ARG;
   c->bgzf_crc = on != 0;
+  return RSIGPU_OK;
+}
+int rsigpu_set_bam_by_ref(rsigpu_ctx* c, int on) {
+  if (!c) return RSIGPU_E_ARG;
+  if (on && c->ix_on) { c->fail("set_bam_by_ref: not available while a BAM index is built (rsigpu_bam_index_begin): the index needs the records in file order"); return RSIGPU_E_ARG; }
+  if (on && c->b_active && c->b_nref > BY_REF_MAX_REFS) {
+    c->fail("set_bam_by_ref: " + std::to_string(c->b_nref) + " references, more than the 65535 that grouping records by refID supports");
+    return RSIGPU_E_ARG;
+  }
+  c->bam_by_ref = on != 0;
   return RSIGPU_OK;
 }
 int rsigpu_set_feed_limit(rsigpu_ctx* c, int64_t decoded_bytes) {

@@ -39,7 +39,7 @@ namespace {
 
 struct Opt {
   std::string function = "rsi", rdfile, bamfile, reffile, cnvfile, outfile = "rsiout.txt", chr = "1-22XY";
-  bool saverd = false, hostdecode = false, crc = false, out_set = false;
+  bool saverd = false, hostdecode = false, crc = false, out_set = false, unsorted = false;
   int gpus = 1, threads = 8, split = 1;
   rsigpu_params P;
 };
@@ -52,7 +52,9 @@ int usage() {
           "   -q  INT  minimum mapping quality [0]\n   -Q  INT  minimum base quality [13]\n   -cap FLT cap depth at FLT x median, <=1 off [4]\n"
           "   -NOGC    no GC adjustment\n   -MED | -NB | -ALL  transformation [NB]\n   -s       save raw depth to <out>.<chr>_rd (BAM input)\n"
           "   -gpus INT  GPUs to shard contigs over [1]\n   -split INT  spread EVERY contig over INT GPUs instead (base ranges + halos, identical table) [1]\n   -hostdecode  inflate/parse the BAM on the host (zlib, -threads INT [8]) instead of on the GPU\n"
-          "   -crc     check the CRC32 of every BGZF block the GPU decodes (the host decoder always does)\n");
+          "   -crc     check the CRC32 of every BGZF block the GPU decodes (the host decoder always does)\n"
+          "   -unsorted  the BAM need not be coordinate-sorted (rsi, stat): records are grouped by contig while decoding and each contig's\n"
+          "              reads sorted on the GPU; every contig's reads stay in GPU memory until the end of the file; the .bai is not read\n");
   return 0;
 }
 
@@ -95,6 +97,7 @@ bool parse(int argc, char** argv, Opt* o) {
     if (k == "-threads") { o->threads = atoi(val(i).c_str()); two(); continue; }
     if (k == "-hostdecode") { o->hostdecode = true; a[i] = ""; continue; }
     if (k == "-crc") { o->crc = true; a[i] = ""; continue; }
+    if (k == "-unsorted") { o->unsorted = true; a[i] = ""; continue; }
   }
   bool bad = false;
   for (size_t i = 1; i < a.size(); ++i) if (!a[i].empty()) { fprintf(stderr, "unknown option %s\n", a[i].c_str()); bad = true; }
@@ -632,6 +635,112 @@ int bam_on_gpu(const Opt& o, const std::vector<std::vector<rsigpu_ctx*>>& ctx, s
   return failed.load() ? 1 : 0;
 }
 
+// `-unsorted`: a BAM in any record order (an aligner's input or name order).  The decoder on GPU 0 groups every feed's records by
+// refID (rsigpu_set_bam_by_ref); each run of an eligible contig is appended to one staging context on the contig's GPU and noted as a
+// (r0, r1) segment of it.  At the end of the file every GPU runs its contigs, its two contexts alternating: the contig's segments
+// are moved over (rsigpu_reads_take), sorted by position, stable in file order (rsigpu_pileup_sort), and run as usual -- what the
+// sorted route computes on the same file after a stable coordinate sort.  Unlike the sorted route, every contig's reads stay in
+// GPU memory until the end of the file.  A contig whose reads could not all be staged, or a file that cannot be read to its end,
+// fails with its name on stderr and no rows: never calls from part of a contig's reads.  The .bai is not read.
+int bam_unsorted_on_gpu(const Opt& o, const std::vector<std::vector<rsigpu_ctx*>>& ctx, std::vector<ContigResult>* results_out) {
+  const bool timing = getenv("RSICNV_TIMING") != nullptr;
+  const double t_start = now_s();
+  std::string err;
+  long long coff = 0, skip = 0;
+  BamHeader h;
+  if (!read_bam_header(o.bamfile, &h, &coff, &skip, &err)) { fprintf(stderr, "%s\n", err.c_str()); return 1; }
+  std::vector<ContigResult>& results = *results_out;
+  results.resize(h.name.size());
+  for (size_t i = 0; i < h.name.size(); ++i) results[i].name = h.name[i];
+  if (o.chr != "1-22XY" && std::find(h.name.begin(), h.name.end(), o.chr) == h.name.end()) { fprintf(stderr, "BAM file doesn't have %s\n", o.chr.c_str()); return 0; }
+  const int ng = (int)ctx.size(), n_ref = (int)h.name.size();
+  const std::vector<int> gpu_of = lpt_assign(o, h, ng, nullptr);
+  std::mutex mu;
+  std::atomic<int> failed(0);
+  auto fail_contig = [&](int tid, const std::string& what) {
+    std::lock_guard<std::mutex> lk(mu);
+    results[(size_t)tid].err = what; results[(size_t)tid].done = false;
+    fprintf(stderr, "%s: %s\n", results[(size_t)tid].name.c_str(), what.c_str());
+    failed++;
+  };
+  std::vector<rsigpu_ctx*> stage((size_t)ng, nullptr);
+  auto destroy_all = [&]() { for (rsigpu_ctx*& s : stage) { rsigpu_destroy(s); s = nullptr; } };
+  for (int g = 0; g < ng; ++g)
+    if (rsigpu_create(g, &o.P, &stage[(size_t)g]) || rsigpu_reads_begin(stage[(size_t)g], 0, 1)) {
+      fprintf(stderr, "cannot create the staging context on GPU %d\n", g); destroy_all(); return 2;
+    }
+  rsigpu_ctx* dec = nullptr;
+  if (create_decoder(o, 0, &dec) || rsigpu_set_bam_by_ref(dec, 1) || rsigpu_bam_begin(dec, (int32_t)n_ref)) {
+    fprintf(stderr, "%s\n", dec ? rsigpu_last_error(dec) : "cannot create the decoder context"); rsigpu_destroy(dec); destroy_all(); return 2;
+  }
+  std::vector<std::vector<std::pair<int64_t, int64_t>>> seg((size_t)n_ref);
+  std::vector<int64_t> staged((size_t)ng, 0);
+  std::vector<std::string> stage_err((size_t)ng);   // non-empty: GPU g's staged reads are incomplete, every contig of it fails
+  DecodeTiming tm;
+  const int rc = stream_bam(o.bamfile, coff, skip, 0, dec, (size_t)256 << 20, [&](int i, const rsigpu_bam_run& run) {
+    if (run.tid < 0 || gpu_of[(size_t)run.tid] < 0) return 0;    // unplaced, or not processed: the file goes on
+    const int g = gpu_of[(size_t)run.tid];
+    if (!stage_err[(size_t)g].empty()) return 0;
+    if (rsigpu_bam_take(dec, i, stage[(size_t)g])) { stage_err[(size_t)g] = rsigpu_last_error(stage[(size_t)g]); return 0; }
+    seg[(size_t)run.tid].emplace_back(staged[(size_t)g], staged[(size_t)g] + run.n_reads);
+    staged[(size_t)g] += run.n_reads;
+    return 0;
+  }, &tm);
+  rsigpu_destroy(dec);
+  const double t_decoded = now_s();
+  for (int t = 0; t < n_ref; ++t) {
+    const int g = gpu_of[(size_t)t];
+    if (g < 0) continue;
+    if (rc) { if (!seg[(size_t)t].empty()) fail_contig(t, "the BAM file could not be decoded to its end: with -unsorted every contig may be incomplete"); }
+    else if (!stage_err[(size_t)g].empty())
+      fail_contig(t, "-unsorted keeps the reads of all contigs of GPU " + std::to_string(g) + " in one staging context until the end of the file, and staging them failed (" +
+                     stage_err[(size_t)g] + "); more GPUs (-gpus) spread them");
+  }
+  if (rc) failed++;
+  std::vector<std::thread> lanes;
+  for (int g = 0; g < ng && !rc; ++g)
+    lanes.emplace_back([&, g]() {
+      std::vector<int> tids;
+      if (stage_err[(size_t)g].empty()) for (int t = 0; t < n_ref; ++t) if (gpu_of[(size_t)t] == g && !seg[(size_t)t].empty()) tids.push_back(t);
+      FastaPrefetch fp(o.reffile);
+      if (!tids.empty()) fp.request(h.name[(size_t)tids[0]]);
+      std::thread fin[2];
+      for (size_t k = 0; k < tids.size(); ++k) {
+        const int tid = tids[k]; const size_t slot = k % ctx[(size_t)g].size();
+        rsigpu_ctx* c = ctx[(size_t)g][slot];
+        if (fin[slot & 1].joinable()) fin[slot & 1].join();
+        ContigResult& r = results[(size_t)tid];
+        { std::lock_guard<std::mutex> lk(mu); fprintf(stderr, "#processing %s on GPU %d\n", r.name.c_str(), g); }
+        std::string fasta, e2;
+        const bool got = fp.take(r.name, &fasta, &e2);
+        if (k + 1 < tids.size()) fp.request(h.name[(size_t)tids[k + 1]]);
+        if (!got) { fail_contig(tid, e2); continue; }
+        if ((int)fasta.size() != h.len[(size_t)tid]) fprintf(stderr, "reference and target not same size %zu\t%d\n", fasta.size(), h.len[(size_t)tid]);
+        if (!begin_contig(c, tid, fasta, nullptr, &r)) { fail_contig(tid, r.err); continue; }
+        std::string what;
+        for (const auto& sg : seg[(size_t)tid])
+          if (rsigpu_reads_take(stage[(size_t)g], sg.first, sg.second, c)) { what = std::string("reads_take: ") + rsigpu_last_error(c); break; }
+        if (what.empty() && rsigpu_pileup_sort(c)) what = std::string("pileup_sort: ") + rsigpu_last_error(c);
+        if (!what.empty()) { fail_contig(tid, what); continue; }
+        const size_t flen = fasta.size();
+        fin[slot & 1] = std::thread([&, c, tid, flen]() {
+          ContigResult& rr = results[(size_t)tid];
+          rr.done = finish_contig(c, o, rr.name, flen, true, &rr);
+          if (!rr.done) { std::lock_guard<std::mutex> lk(mu); fprintf(stderr, "%s: %s\n", rr.name.c_str(), rr.err.c_str()); failed++; }
+        });
+      }
+      for (auto& f : fin) if (f.joinable()) f.join();
+    });
+  for (auto& l : lanes) l.join();
+  destroy_all();
+  if (timing) {
+    int64_t total = 0; for (int64_t x : staged) total += x;
+    fprintf(stderr, "#timing: -unsorted decode + staging %.3f s (%lld reads staged; first read %.3f, bam_feed %.3f, take %.3f), contigs %.3f s\n",
+            t_decoded - t_start, (long long)total, tm.read, tm.feed, tm.take, now_s() - t_decoded);
+  }
+  return failed.load() ? 1 : 0;
+}
+
 // `rsicnv stat -b BAM -v CNVFILE -o OUT` (rsi.cpp:2235-2249): every line of CNVFILE that names a call (read_cnvlist,
 // loaddata.cpp:606-673: >= 5 characters, not a comment, >= 4 fields RNAME START END TYPE) is written back followed by
 // RP=<supporting read pairs>;Q0=<fraction of mapq-0 reads> (cnv_stat, pairrd.cpp:622-748).  The reads of every contig that
@@ -676,7 +785,33 @@ int do_stat(const Opt& o, rsigpu_ctx* c) {
   auto stat_contig = [&](int tid) {
     if (rsigpu_stat_calls(c, list.data(), (int32_t)list.size())) { fprintf(stderr, "%s: %s\n", h.name[(size_t)tid].c_str(), rsigpu_last_error(c)); ++failed; }
   };
-  if (indexed) {
+  if (o.unsorted) {   // records grouped by refID while decoding into one staging context, then per contig moved over and sorted
+    rsigpu_ctx* stage = nullptr;
+    if (rsigpu_create(0, &o.P, &stage) || rsigpu_reads_begin(stage, 0, 1) || rsigpu_set_bam_by_ref(dec, 1) || rsigpu_bam_begin(dec, (int32_t)n_ref)) {
+      fprintf(stderr, "%s\n", stage ? rsigpu_last_error(dec) : "cannot create the staging context"); rsigpu_destroy(stage); rsigpu_destroy(dec); return 2;
+    }
+    std::vector<std::vector<std::pair<int64_t, int64_t>>> seg((size_t)n_ref);
+    int64_t staged = 0; std::string stage_err;
+    const int rc = stream_bam(o.bamfile, coff, skip, 0, dec, (size_t)256 << 20, [&](int i, const rsigpu_bam_run& run) {
+      if (run.tid < 0 || !wanted[(size_t)run.tid] || !stage_err.empty()) return 0;
+      if (rsigpu_bam_take(dec, i, stage)) { stage_err = rsigpu_last_error(stage); return 0; }
+      seg[(size_t)run.tid].emplace_back(staged, staged + run.n_reads); staged += run.n_reads;
+      return 0;
+    }, &tm);
+    if (rc) ++failed;
+    else if (!stage_err.empty()) { fprintf(stderr, "-unsorted keeps the reads of every contig with calls in one staging context until the end of the file, and staging them failed (%s)\n", stage_err.c_str()); ++failed; }
+    else
+      for (int tid = 0; tid < n_ref; ++tid) {
+        if (seg[(size_t)tid].empty()) continue;
+        fprintf(stderr, "#sampling %s\n", h.name[(size_t)tid].c_str());
+        bool ok = rsigpu_reads_begin(c, tid, h.len[(size_t)tid]) == 0;
+        for (size_t k = 0; ok && k < seg[(size_t)tid].size(); ++k) ok = rsigpu_reads_take(stage, seg[(size_t)tid][k].first, seg[(size_t)tid][k].second, c) == 0;
+        if (ok) ok = rsigpu_pileup_sort(c) == 0;
+        if (!ok) { fprintf(stderr, "%s: %s\n", h.name[(size_t)tid].c_str(), rsigpu_last_error(c)); ++failed; continue; }
+        stat_contig(tid);
+      }
+    rsigpu_destroy(stage);
+  } else if (indexed) {
     for (int tid = 0; tid < n_ref; ++tid) {
       if (!wanted[(size_t)tid] || !bai[(size_t)tid].has_reads) continue;
       fprintf(stderr, "#sampling %s\n", h.name[(size_t)tid].c_str());
@@ -815,6 +950,7 @@ int main(int argc, char** argv) {
   Opt o;
   if (!parse(argc, argv, &o)) return usage();
   if (o.function == "decode") return do_decode(o);
+  if (o.unsorted && (o.split > 1 || o.hostdecode)) { fprintf(stderr, "-unsorted works with the GPU decoder and without -split\n"); return 2; }
   const double t_main = now_s();
   const int ndev = rsigpu_num_devices();
   if (ndev <= 0) { fprintf(stderr, "no CUDA device: this implementation has no CPU path\n"); return 2; }
@@ -862,6 +998,9 @@ int main(int argc, char** argv) {
     std::vector<rsigpu_ctx*> parts;
     for (int g = 0; g < ng; ++g) parts.push_back(ctx[(size_t)g][0]);
     rc_all = bam_split_on_gpu(o, parts, &results);
+    if (rc_all == 2) return 2;
+  } else if (o.unsorted) {
+    rc_all = bam_unsorted_on_gpu(o, ctx, &results);
     if (rc_all == 2) return 2;
   } else if (!o.hostdecode) {
     rc_all = bam_on_gpu(o, ctx, &results);
@@ -912,7 +1051,7 @@ int main(int argc, char** argv) {
       BamHeader h; long long co = 0, sk = 0; std::string e3;
       if (read_bam_header(o.bamfile, &h, &co, &sk, &e3)) {
         std::vector<BaiRef> bai;
-        const bool have_idx = read_bai(o.bamfile, h.name.size(), &bai);
+        const bool have_idx = !o.unsorted && read_bai(o.bamfile, h.name.size(), &bai);
         check = "#Check bam header for 1-22XY \n";
         std::string pop = "#BAM has reads on :";
         for (size_t i = 0; i < h.name.size(); ++i) {

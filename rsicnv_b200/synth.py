@@ -468,34 +468,28 @@ def _bam_records(R: dict, tid: int, lo: int, hi: int, random_seq, rich=None, wan
     return buf.tobytes()
 
 
-def write_bam(path: str, contigs: list[tuple[str, int]], reads_by_tid: dict[int, dict], level: int = 1, strategy: int = 0,
-              block_size: int = 65280, random_seq: int | None = None, threads: int = 8, rich: int | None = None,
-              unmapped_tail: int = 0) -> None:
-    """Minimal BAM (BGZF) writer for the synthetic reads: one record per read, name 'r', sequence all 'A'
-    (the path never looks at bases; random_seq=SEED writes random bases instead, which makes the file compress like a
-    real one), qualities as given.  strategy: zlib strategy (zlib.Z_FIXED forces fixed-Huffman blocks), level 0 writes
-    stored blocks; records are NOT aligned to BGZF blocks.  Reads are serialised in slabs and the blocks compressed on a
-    thread pool, so a chr19-sized file takes about a minute.  rich=SEED writes real-looking records (names, bases, optional
-    fields); unmapped_tail appends that many refID -1 records.  Layout: SURVEY.md Appendix B."""
+def _bam_header(contigs: list[tuple[str, int]], sort_order: str) -> bytes:
     import struct
-    import zlib
-    from concurrent.futures import ThreadPoolExecutor
-    text = "@HD\tVN:1.0\tSO:coordinate\n" + "".join(f"@SQ\tSN:{n}\tLN:{l}\n" for n, l in contigs)
+    text = f"@HD\tVN:1.0\tSO:{sort_order}\n" + "".join(f"@SQ\tSN:{n}\tLN:{l}\n" for n, l in contigs)
     hdr = bytearray(b"BAM\x01") + struct.pack("<i", len(text)) + text.encode() + struct.pack("<i", len(contigs))
     for n, l in contigs:
         hdr += struct.pack("<i", len(n) + 1) + n.encode() + b"\x00" + struct.pack("<i", l)
+    return bytes(hdr)
 
-    def pieces():
-        yield bytes(hdr)
-        for tid in sorted(reads_by_tid):
-            R = reads_by_tid[tid]
-            nr = len(R["pos"])
-            for lo in range(0, nr, 1 << 19):
-                yield _bam_records(R, tid, lo, min(nr, lo + (1 << 19)), random_seq, rich)
-        for u in range(unmapped_tail):    # unplaced, unmapped reads: refID -1, pos -1, flag 4, no CIGAR
-            name = b"unm%d\x00" % u
-            body = struct.pack("<iiIIiiii", -1, -1, (4680 << 16) | len(name), (4 << 16), 10, -1, -1, 0) + name + b"\x11" * 5 + b"\x1e" * 10
-            yield struct.pack("<I", len(body)) + body
+
+def _unplaced_record(u: int) -> bytes:
+    """an unplaced, unmapped read: refID -1, pos -1, flag 4, no CIGAR"""
+    import struct
+    name = b"unm%d\x00" % u
+    body = struct.pack("<iiIIiiii", -1, -1, (4680 << 16) | len(name), (4 << 16), 10, -1, -1, 0) + name + b"\x11" * 5 + b"\x1e" * 10
+    return struct.pack("<I", len(body)) + body
+
+
+def _write_bgzf(path: str, pieces, level: int, strategy: int, block_size: int, threads: int) -> None:
+    """the concatenated pieces as BGZF blocks of block_size decoded bytes, then the EOF marker"""
+    import struct
+    import zlib
+    from concurrent.futures import ThreadPoolExecutor
 
     def bgzf(blk: bytes) -> bytes:
         co = zlib.compressobj(level, zlib.DEFLATED, -15, 8, strategy)
@@ -505,7 +499,7 @@ def write_bam(path: str, contigs: list[tuple[str, int]], reads_by_tid: dict[int,
     BS = block_size
     with open(path, "wb") as f, ThreadPoolExecutor(threads) as pool:
         carry = b""
-        for piece in pieces():
+        for piece in pieces:
             data = carry + piece
             nfull = len(data) // BS * BS
             for out in pool.map(bgzf, (data[a:a + BS] for a in range(0, nfull, BS))):
@@ -514,6 +508,60 @@ def write_bam(path: str, contigs: list[tuple[str, int]], reads_by_tid: dict[int,
         if carry:
             f.write(bgzf(carry))
         f.write(bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000"))
+
+
+def write_bam(path: str, contigs: list[tuple[str, int]], reads_by_tid: dict[int, dict], level: int = 1, strategy: int = 0,
+              block_size: int = 65280, random_seq: int | None = None, threads: int = 8, rich: int | None = None,
+              unmapped_tail: int = 0) -> None:
+    """Minimal BAM (BGZF) writer for the synthetic reads: one record per read, name 'r', sequence all 'A'
+    (the path never looks at bases; random_seq=SEED writes random bases instead, which makes the file compress like a
+    real one), qualities as given.  strategy: zlib strategy (zlib.Z_FIXED forces fixed-Huffman blocks), level 0 writes
+    stored blocks; records are NOT aligned to BGZF blocks.  Reads are serialised in slabs and the blocks compressed on a
+    thread pool, so a chr19-sized file takes about a minute.  rich=SEED writes real-looking records (names, bases, optional
+    fields); unmapped_tail appends that many refID -1 records.  Layout: SURVEY.md Appendix B."""
+    def pieces():
+        yield _bam_header(contigs, "coordinate")
+        for tid in sorted(reads_by_tid):
+            R = reads_by_tid[tid]
+            nr = len(R["pos"])
+            for lo in range(0, nr, 1 << 19):
+                yield _bam_records(R, tid, lo, min(nr, lo + (1 << 19)), random_seq, rich)
+        for u in range(unmapped_tail):
+            yield _unplaced_record(u)
+    _write_bgzf(path, pieces(), level, strategy, block_size, threads)
+
+
+def write_bam_unsorted(path: str, contigs: list[tuple[str, int]], reads_by_tid: dict[int, dict], order, level: int = 1,
+                       strategy: int = 0, block_size: int = 65280, random_seq: int | None = None, threads: int = 8,
+                       rich: int | None = None) -> None:
+    """write_bam with the records in any interleaving, header `@HD SO:unsorted`.  order: a sequence of refIDs, one per record;
+    the k-th occurrence of refID t writes reads_by_tid[t]'s read k (so each contig's reads appear in the order of its dict,
+    which need not be by position), and each -1 writes the next unplaced, unmapped record (refID -1, pos -1, flag 4)."""
+    order = np.asarray(order, np.int64)
+    tids = sorted(reads_by_tid)
+    for t in tids:
+        assert int(np.count_nonzero(order == t)) == len(reads_by_tid[t]["pos"]), f"order must name refID {t} once per read"
+    assert set(np.unique(order).tolist()) <= set(tids) | {-1}
+    bufs, starts, lens, base = [], {}, {}, 0
+    for t in tids:
+        b, offs = _bam_records(reads_by_tid[t], t, 0, len(reads_by_tid[t]["pos"]), random_seq, rich, want_offsets=True)
+        bufs.append(np.frombuffer(b, np.uint8)); starts[t] = base + offs[:-1]; lens[t] = np.diff(offs); base += len(b)
+    n_un = int(np.count_nonzero(order == -1))
+    un = [_unplaced_record(u) for u in range(n_un)]
+    ul = np.array([len(r) for r in un], np.int64)
+    bufs.append(np.frombuffer(b"".join(un), np.uint8)); starts[-1] = base + np.concatenate(([0], np.cumsum(ul)[:-1])) if n_un else np.zeros(0, np.int64); lens[-1] = ul
+    src = np.concatenate(bufs) if bufs else np.zeros(0, np.uint8)
+    rec_start = np.zeros(len(order), np.int64); rec_len = np.zeros(len(order), np.int64)
+    for t in list(tids) + [-1]:
+        at = np.flatnonzero(order == t)
+        rec_start[at] = starts[t]; rec_len[at] = lens[t]
+    body = src[np.repeat(rec_start, rec_len) + (np.arange(int(rec_len.sum())) - np.repeat(np.cumsum(rec_len) - rec_len, rec_len))]
+
+    def pieces():
+        yield _bam_header(contigs, "unsorted")
+        for a in range(0, len(body), 1 << 26):
+            yield body[a:a + (1 << 26)].tobytes()
+    _write_bgzf(path, pieces(), level, strategy, block_size, threads)
 
 
 def write_bam_aligned(path: str, name: str, L: int, reads: dict, level: int = 1, random_seq: int | None = None, threads: int = 8,
