@@ -31,13 +31,17 @@ struct ReadSoA {
 };
 __device__ __forceinline__ int read_ncig(const ReadSoA& R, i64 r) { return R.cigar_off ? (int)(R.cigar_off[r + 1] - R.cigar_off[r]) : (int)R.ncig[r]; }
 enum { BF_PROPER = 2, BF_REV = 16, BF_MREV = 32, BF_SECONDARY = 256, BF_DUP = 1024 };
-enum { PU_T = 8192, PU_NT = 256 };
+// PU_T: positions per tile of k_pileup_tile.  4096 keeps the shared difference array at 17 KB, so 8 blocks of PU_NT
+// threads fit an SM (full occupancy at 32 registers; 8192 held it to 6 blocks).  PU_ENDS_PER_SM: read-end blocks per SM
+// in k_qual_mask.
+enum { PU_T = 4096, PU_NT = 256, PU_ENDS_PER_SM = 4 };
 
 // per read: bam_calend, and the largest reference extent any of its counted bases can reach
-// (reference coordinates advance on M, D, N and S from the first M/D/=/X op: samfunctions.cpp:59-100)
-__global__ void k_read_ends(ReadSoA R, int* max_extent, int* sorted_bad) {
+// (reference coordinates advance on M, D, N and S from the first M/D/=/X op: samfunctions.cpp:59-100).
+// Reads r0, r0 + stride, ...: the body of k_read_ends and of the read-end blocks of k_qual_mask.
+__device__ __forceinline__ void read_ends_body(const ReadSoA& R, i64 r0, i64 stride, int* max_extent, int* sorted_bad) {
   int mx = 0, bad = 0;
-  for (i64 r = (i64)blockIdx.x * blockDim.x + threadIdx.x; r < R.n; r += (i64)gridDim.x * blockDim.x) {
+  for (i64 r = r0; r < R.n; r += stride) {
     const u32 c0 = R.cigar_off[r], c1 = R.cigar_off[r + 1];
     u32 end = (u32)R.pos[r], ext = 0; bool anchored = false;
     for (u32 k = c0; k < c1; ++k) {
@@ -58,6 +62,9 @@ __global__ void k_read_ends(ReadSoA R, int* max_extent, int* sorted_bad) {
   if (mx) atomicMax(max_extent, mx);
   if (bad) atomicOr(sorted_bad, 1);
 }
+__global__ void k_read_ends(ReadSoA R, int* max_extent, int* sorted_bad) {
+  read_ends_body(R, (i64)blockIdx.x * blockDim.x + threadIdx.x, (i64)gridDim.x * blockDim.x, max_extent, sorted_bad);
+}
 
 // Base-quality filter as a pure streaming pass: one bit per quality byte (bit i of word w = byte 32w+i has
 // quality >= Q), 32 bytes per thread, SWAR byte compare (exact for any Q in [0, 255]; Q > 255 passes nothing).
@@ -67,12 +74,20 @@ __device__ __forceinline__ u32 qual_pass_nibble(u32 w, u32 qlow4, bool qhigh) {
   const u32 m7 = (qhigh ? (w & t) : (w | t)) & 0x80808080u;
   return ((m7 >> 7) * 0x01020408u) >> 24;
 }
-__global__ void __launch_bounds__(256) k_qual_mask(const u8* __restrict__ qual, u64 nbytes, int min_baseQ, u32* __restrict__ mask) {
+// Blocks [0, nb_ends) run the read-end pass (read_ends_body) over all reads, the others stream the quality bytes: the
+// latency-bound CIGAR walk runs on the same SMs as the bandwidth-bound stream instead of alone before it.
+__global__ void __launch_bounds__(256) k_qual_mask(const u8* __restrict__ qual, u64 nbytes, int min_baseQ, u32* __restrict__ mask,
+                                                   ReadSoA R, int* max_extent, int* sorted_bad, int nb_ends) {
+  if ((int)blockIdx.x < nb_ends) {
+    read_ends_body(R, (i64)blockIdx.x * blockDim.x + threadIdx.x, (i64)nb_ends * blockDim.x, max_extent, sorted_bad);
+    return;
+  }
   const int Qc = min_baseQ < 0 ? 0 : min_baseQ;
   const bool q_none = Qc > 255, qhigh = Qc > 128;
   const u32 qlow4 = (u32)(qhigh ? Qc - 128 : Qc) * 0x01010101u;
   const u64 nwords = (nbytes + 31) >> 5;
-  for (u64 w = (u64)blockIdx.x * blockDim.x + threadIdx.x; w < nwords; w += (u64)gridDim.x * blockDim.x) {
+  const u64 stride = (u64)(gridDim.x - nb_ends) * blockDim.x;
+  for (u64 w = (u64)(blockIdx.x - nb_ends) * blockDim.x + threadIdx.x; w < nwords; w += stride) {
     const uint4 a = reinterpret_cast<const uint4*>(qual)[2 * w], b = reinterpret_cast<const uint4*>(qual)[2 * w + 1];
     u32 m = qual_pass_nibble(a.x, qlow4, qhigh) | (qual_pass_nibble(a.y, qlow4, qhigh) << 4) | (qual_pass_nibble(a.z, qlow4, qhigh) << 8) |
             (qual_pass_nibble(a.w, qlow4, qhigh) << 12) | (qual_pass_nibble(b.x, qlow4, qhigh) << 16) | (qual_pass_nibble(b.y, qlow4, qhigh) << 20) |
